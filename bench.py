@@ -28,7 +28,11 @@ Prints ONE JSON line (rank 0).  Every key describes the SAME timed arm unless it
   oracle/ref_shim.py) on the host cores: its three calls energy_from_kappa + analytic_gradient +
   analytic_hessian at N = 96 with the workload's CAS, extrapolated to N = 256 by its own flop count (the
   reference cannot run at N = 256: a dozen N^4 tensors); ``cpu_baseline_measured``: a same-config measurement
-  of both implementations at the largest BASELINE config the reference can run (114 AOs, CAS(6,6)).
+  of both implementations at the largest BASELINE config the reference can run (114 AOs, CAS(6,6)).  The
+  reference is not part of this repository: without it both are null and ``cpu_baseline_unavailable`` says why.
+
+``--dump-outputs DIR`` writes the results of the last timed step as float64 ``DIR/<name>.npy`` (see
+``dump_outputs``), so that two builds can be compared on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -49,10 +53,12 @@ F64 = torch.float64
 METRIC = "oo_energy_gradient_hessian_evals_per_sec"
 UNIT = "evals/s"
 # the CPU reference runs the workload's CAS at this basis size whatever --steps / --warmup are (N=256 cannot run
-# on a host); one E+G+H sample is 10-15 s on 16 cores.  Long runs cap the number of repetitions instead.
+# on a host); one E+G+H sample is 10-15 s on 16 cores.  The budget caps the warm-up repetitions.
 CPU_SAMPLE_NAO = int(os.environ.get("OO_BENCH_CPU_SAMPLE_NAO", "96"))
 CPU_BUDGET_S = float(os.environ.get("OO_BENCH_CPU_BUDGET_S", "150"))
 MEASURED_WORKLOAD = "c6h6_ccpvdz_cas66"           # same-config secondary: the reference can run this one
+DUMP_H_ENTRIES = 1 << 22                          # Hessian entries --dump-outputs keeps over the whole batch (32 MB)
+DUMP_MAX_BYTES = 64 << 20
 
 
 # --------------------------------------------------------------------------------------
@@ -146,6 +152,28 @@ def hbm_peak_gbs():
         return 6553.3, "fallback (MEASURED_PEAKS.json absent): 6553.3 GB/s measured on this pool in round 1"
 
 
+def dump_outputs(out_dir, E, G, H):
+    """Writes one step's results (B evaluations) as float64 ``out_dir/<name>.npy``: ``E`` (B,), the packed gradient
+    ``G`` (B, n_kappa), the Hessian diagonal ``H_diag`` (B, n_kappa) and ``H_sample`` (B, S), the Hessian entries at
+    S flat positions of the n_kappa x n_kappa matrix drawn once from a fixed seed (the same positions in every
+    evaluation and every run; all entries, in order, when they fit DUMP_H_ENTRIES)."""
+    import numpy as np
+    B, nk = G.shape
+    n = min(nk * nk, DUMP_H_ENTRIES // B)
+    if n == nk * nk:
+        idx = torch.arange(n)
+    else:
+        idx = torch.randint(nk * nk, (n,), generator=torch.Generator().manual_seed(0)).sort().values
+    arrays = {"E": E, "G": G, "H_diag": H.diagonal(dim1=1, dim2=2),
+              "H_sample": H.reshape(B, nk * nk)[:, idx.to(H.device)]}
+    arrays = {k: v.detach().to("cpu", F64).contiguous().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------
 # CPU arm: the verbatim reference behind the pennylane.math shim
 # --------------------------------------------------------------------------------------
@@ -191,12 +219,12 @@ def cpu_reference_sample(shape_name, nao_sample, reps=1):
     best = float("inf")
     for _ in range(reps):
         t0 = time.perf_counter()
-        reference_evaluation(oo, one, two, kappa)
+        outputs = reference_evaluation(oo, one, two, kappa)
         best = min(best, time.perf_counter() - t0)
     flops = lambda n: 24.0 * n ** 5 + 6.0 * n ** 6
     scale = flops(nao) / flops(ns)
     return {"seconds_sample": best, "nao_sample": ns, "scale": scale, "cores": cores,
-            "evals_per_s": 1.0 / (best * scale)}
+            "evals_per_s": 1.0 / (best * scale), "outputs": outputs}
 
 
 def cpu_baseline_dict(r, nao):
@@ -222,8 +250,8 @@ def run_reference(args, rank, world):
     per = first["seconds_sample"]
     for _ in range(min(max(args.warmup, 1) - 1, max(0, int(0.2 * CPU_BUDGET_S / per)))):
         cpu_reference_sample(args.workload, CPU_SAMPLE_NAO)
-    # same sample size whatever --steps is; a long run repeats fewer times than it reports steps
-    measured = max(1, min(args.steps, int(CPU_BUDGET_S / per)))
+    # same sample size whatever --steps is; every step is one evaluation of that sample
+    measured = args.steps
     wall, res = 0.0, None
     for _ in range(measured):
         res = cpu_reference_sample(args.workload, CPU_SAMPLE_NAO)
@@ -241,6 +269,9 @@ def run_reference(args, rank, world):
         "cpu_baseline": cpu,
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        E, G, H = (torch.as_tensor(x)[None] for x in res["outputs"])
+        dump_outputs(args.dump_outputs, E, G, H)
     print(json.dumps(line), flush=True)
 
 
@@ -323,7 +354,7 @@ def strong_arm(args, mol, ncas, nelecas, dev, world, rank, n_evals, max_over_ran
     checks = (E[0].item(), G[0].clone(), H[0].diagonal().sum().item())
     del oo, eng
     torch.cuda.empty_cache()
-    return out, checks
+    return out, checks, (E, G, H)
 
 
 # --------------------------------------------------------------------------------------
@@ -343,7 +374,12 @@ def main():
                          "every evaluation is spread over all GPUs (OO_energy(shard='pairs')); with --mode weak and "
                          "N > 1 a short strong-mode arm is reported as well under `strong_scaling`")
     ap.add_argument("--strong-evals", type=int, default=6)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's E, gradient, Hessian diagonal and a seeded "
+                         "sample of Hessian entries as float64 DIR/<name>.npy (rank 0; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                                   # timing rule: W >= 3
     rank, world, local = dist_env()
@@ -401,10 +437,12 @@ def main():
         if rank == 0:
             sampler.start()
         launches0 = lib.oo_launch_count()
-        strong, _ = strong_arm(args, mol, ncas, nelecas, dev, world, rank, max(args.steps, 1) * B, max_over_ranks,
-                               barrier)
+        strong, _, last = strong_arm(args, mol, ncas, nelecas, dev, world, rank, args.steps * B, max_over_ranks,
+                                     barrier)
         launches = lib.oo_launch_count() - launches0
         clocks = sampler.stop() if rank == 0 else None
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, *last)
         if rank == 0:
             line = {"metric": METRIC, "value": strong["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
                     "warmup": 3, "ms_per_step": strong["ms_per_evaluation"] * B, "higher_is_better": True,
@@ -488,6 +526,8 @@ def main():
     t_dev = max_over_ranks(t_local)
     checksum = float(E.sum().item() + G.abs().sum().item() + H.diagonal(dim1=1, dim2=2).sum().item())
     E_dev_last, G_dev_last, H_dev_last = E.clone(), G.clone(), H[-1].clone()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, E, G, H)
     if full_arm is not None:                              # both formulations must agree on the last step's results
         assert (E - full_arm["E"]).abs().max().item() < 1e-9 and (G - full_arm["G"]).abs().max().item() < 1e-8
         assert abs(H.diagonal(dim1=1, dim2=2).sum().item() - full_arm["h_diag"]) < 1e-6
@@ -609,7 +649,8 @@ def main():
     if want_strong:
         eng.release_workspaces()
         torch.cuda.empty_cache()
-        strong, chk = strong_arm(args, mol, ncas, nelecas, dev, world, rank, args.strong_evals, max_over_ranks, barrier)
+        strong, chk, _ = strong_arm(args, mol, ncas, nelecas, dev, world, rank, args.strong_evals, max_over_ranks,
+                                    barrier)
         strong["one_gpu_ms_per_evaluation_same_run"] = t_dev / (B * args.steps) * 1e3
         strong["speedup_vs_one_gpu"] = strong["one_gpu_ms_per_evaluation_same_run"] / strong["ms_per_evaluation"]
         mol._B = None
@@ -696,8 +737,12 @@ def main():
                          "evals_per_s": world * n_evals / full_arm["t"],
                          "measured_on": "its own arm (path='full'), not the arm that produces `value`"}
 
-    cpu = cpu_measured = None
-    if not args.no_cpu_baseline:
+    from oracle.ref_shim import reference_available
+    cpu = cpu_measured = cpu_unavailable = None
+    if not args.no_cpu_baseline and not reference_available():
+        cpu_unavailable = ("not measured: the auto_oo reference sources are not installed (AUTO_OO_REFERENCE, or "
+                           "baseline/_ref; see oracle/ref_shim.py)")
+    elif not args.no_cpu_baseline:
         cpu_reference_sample(args.workload, CPU_SAMPLE_NAO)                # warm-up (thread pool, allocator)
         cpu = cpu_baseline_dict(cpu_reference_sample(args.workload, CPU_SAMPLE_NAO, reps=2), nao)   # best of two
         if args.workload == "synthetic_n256_cas1212":
@@ -721,7 +766,7 @@ def main():
         "e2e": e2e, "e2e_dense": e2e_dense, "e2e_newton": e2e_newton, "strong_scaling": strong,
         "gpu_launches": int(launches), "clocks": clocks, "roofline": roofline, "roofline_kernels": kernel_rows,
         "roofline_hbm": roofline_hbm, "roofline_full_transform": roofline_full, "stage_ms_per_evaluation": stage_ms,
-        "cpu_baseline": cpu, "cpu_baseline_measured": cpu_measured,
+        "cpu_baseline": cpu, "cpu_baseline_measured": cpu_measured, "cpu_baseline_unavailable": cpu_unavailable,
         "transform_tflops": None if roofline_full is None else roofline_full["achieved"],
         "checksum": checksum,
     }
