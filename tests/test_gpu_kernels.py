@@ -41,6 +41,11 @@ def _stream():
 @pytest.mark.parametrize("M,N,K,batch", [
     (64, 64, 64, 1), (130, 7, 9, 1), (257, 33, 50, 1), (1000, 114, 114, 1), (343, 8, 8, 3),
     (28 ** 3, 28, 28, 2), (100, 484, 201, 1), (576, 12996 // 4, 1153, 1),
+    # 17-24 and 41-48 columns (the 24- and 48-wide tiles), 129-192 rows by >= 9472 columns (the 192-row tile); K = 1, 7,
+    # 9, 15 mod 16 ends on a partial k-block
+    (300, 20, 64, 2), (300, 20, 33, 2), (300, 20, 39, 2), (300, 20, 41, 2), (300, 20, 47, 2), (513, 45, 72, 1),
+    (129, 42, 23, 3), (176, 9472, 64, 1), (176, 9472, 49, 1), (176, 9472, 55, 1), (176, 9476, 57, 1),
+    (176, 9472, 63, 1),
 ])
 def test_dgemm_tn(lib, M, N, K, batch):
     gen = torch.Generator(device="cuda").manual_seed(M * 7 + N)
@@ -653,37 +658,51 @@ def test_unusual_orbital_spaces_against_the_oracle(nao, nelec, ncas, nelecas, fr
 
 
 @pytest.mark.parametrize("nao,nelec,ncas,nelecas", [(64, 64, 4, 4), (70, 100, 6, 6), (56, 36, 4, 4), (60, 60, 4, 4),
-                                                    (57, 44, 6, 6), (129, 40, 4, 4)])
+                                                    (57, 44, 6, 6), (129, 40, 4, 4), (40, 32, 4, 4), (60, 80, 4, 4),
+                                                    (62, 80, 6, 6), (64, 84, 6, 6), (64, 88, 6, 6)])
 def test_class_transform_with_wide_class_index(nao, nelec, ncas, nelecas):
     """Class index nIp in (16, 64]: exercises the 24/32/40/48/64-wide GEMM tiles, every triangular quarter-2
-    configuration (nI = 20, 32, 34; 54 takes the rectangular GEMM), an odd basis size and, at 129 orbitals, the staged
-    128 x 128 class-expand epilogue with a ragged edge (small fixtures only reach the 16-wide tile).  Class tensors must equal slices of the full transform,
-    and E / G / H of both paths must agree."""
+    configuration (nI = 18, 20, 32, 34, 42 .. 47; 54 takes the rectangular GEMM), an odd basis size and, at 129
+    orbitals, the staged 128 x 128 class-expand epilogue with a ragged edge (small fixtures only reach the 16-wide
+    tile).  A batch of three kappas: where nIp is 18 .. 24 or 42 .. 48 the first two share one quarter-1 GEMM (36 .. 48
+    or 84 .. 96 columns) and the third runs alone.  Class tensors must equal slices of the full transform, E / G / H
+    of both paths must agree, and every member must match the CPU class oracle."""
     from auto_oo_b200.engine import HotPathEngine
     from auto_oo_b200.synthetic import SyntheticMol, random_rdms, random_kappa
+    from oracle import class_oracle
     from oracle import oo_oracle as orc
     mol = SyntheticMol(nao, nelec, seed=11)
     occ, act, virt = mol.get_active_space_idx(ncas, nelecas)
     pidx = orc.non_redundant_indices(occ, act, virt, False)
     eng = HotPathEngine(mol.int1e_ao, mol.int2e_ao, mol.oao_coeff, mol.nuc, nao, len(occ), ncas, pidx)
     one, two = random_rdms(ncas, nelecas, seed=2)
-    kap = random_kappa(len(pidx), seed=2, scale=0.05)[None]
+    k0 = random_kappa(len(pidx), seed=2, scale=0.05)
+    kap = torch.stack([k0, random_kappa(len(pidx), seed=3, scale=0.05), -0.5 * k0])
     Coao = eng.to_padded(mol.random_oao_mo_coeff, 2)
     C = eng.mo_coeff(Coao, eng.rotation(kap))
-    cls = eng.class_integrals(C[0])[0]
-    g = eng.int2e_transform(C)[0]
+    cls = eng.class_integrals(C)
+    g = eng.int2e_transform(C)
     nI, nIp, ld = eng.nI, eng.nIp, eng.ld
-    K = cls[:nIp * nIp].reshape(nIp, nIp, ld, ld)[:nI, :nI]
-    J = cls[nIp * nIp:2 * nIp * nIp].reshape(nIp, nIp, ld, ld)[:nI, :nI]
-    assert (J - g[:, :, :nI, :nI].permute(2, 3, 0, 1)).abs().max().item() < 1e-10
-    assert (K - g[:, :nI, :nI, :].permute(2, 1, 0, 3)).abs().max().item() < 1e-10
+    for b in range(3):
+        K = cls[b, :nIp * nIp].reshape(nIp, nIp, ld, ld)[:nI, :nI]
+        J = cls[b, nIp * nIp:2 * nIp * nIp].reshape(nIp, nIp, ld, ld)[:nI, :nI]
+        assert (J - g[b][:, :, :nI, :nI].permute(2, 3, 0, 1)).abs().max().item() < 1e-10, b
+        assert (K - g[b][:, :nI, :nI, :].permute(2, 1, 0, 3)).abs().max().item() < 1e-10, b
+    del cls, g
     Ec, Gc, Hc = eng.evaluate(Coao, one, two, kappa=kap, path="class")
     Ef, Gf, Hf = eng.evaluate(Coao, one, two, kappa=kap, path="full")
-    assert abs(Ec.item() - Ef.item()) < TOL_E
+    assert (Ec - Ef).abs().max().item() < TOL_E
     assert (Gc - Gf).abs().max().item() < TOL_GH and (Hc - Hf).abs().max().item() < TOL_GH
+    ref = class_oracle.ClassProblem(mol.int1e_ao, mol.int2e_ao, mol.oao_coeff, mol.random_oao_mo_coeff, mol.nuc,
+                                    nelec, ncas, nelecas, False)
+    for b in range(3):
+        Eo, Go, Ho = ref.evaluate(one, two, kap[b])
+        assert abs(Ec[b].item() - Eo.item()) < TOL_E, b
+        assert (Gc[b].cpu() - Go).abs().max().item() < TOL_GH, b
+        assert (Hc[b].cpu() - Ho).abs().max().item() < TOL_GH, b
     prob = orc.OracleProblem(mol.int1e_ao, mol.int2e_ao, mol.oao_coeff, mol.random_oao_mo_coeff, mol.nuc,
                              nelec, ncas, nelecas, False)
-    assert abs(Ec.item() - prob.energy(one, two, kap[0]).item()) < TOL_E
+    assert abs(Ec[0].item() - prob.energy(one, two, kap[0]).item()) < TOL_E
     assert (Gc[0].cpu() - prob.gradient(one, two, kap[0])).abs().max().item() < TOL_GH
 
 
