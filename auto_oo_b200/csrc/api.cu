@@ -20,6 +20,9 @@ size_t class_transform_ws_bytes(int ld, int nIp, int batch);
 size_t class_buffer_bytes(int ld, int nIp);
 size_t class_transform_sym_ws_bytes(int ld, int nIp, int batch);
 size_t class_hessian_ws_bytes(int ld, int nIp, int no, int na, int batch);
+size_t class_hessian_vector_ws_bytes(int ld, int nIp, int no, int na, int nv);
+size_t hessian_vector_ws_bytes(int ld, int nI, int na, int nv);
+size_t hessian_diagonal_ws_bytes(int ld, int nI);
 
 int sm_count() {
     static int cached[64] = {};                         // per device
@@ -161,6 +164,11 @@ size_t oo_workspace_bytes(int which, int N, int ld, int nI, int batch) {
         case OO_WS_CLASS_BUFFER: return (size_t)batch * oo::class_buffer_bytes(ld, nI + (nI & 1));
         case OO_WS_CLASS_HESSIAN:   /* N carries na here (the sparse layout depends on no, na, not on N) */
             return oo::class_hessian_ws_bytes(ld, nI + (nI & 1), nI - N, N, batch);
+        case OO_WS_CLASS_HESSIAN_VECTOR:   /* N carries na, batch the number of vectors */
+            return (N > 0 && N <= nI) ? oo::class_hessian_vector_ws_bytes(ld, nI + (nI & 1), nI - N, N, batch) : 0;
+        case OO_WS_HESSIAN_VECTOR:
+            return (N > 0 && N <= nI) ? oo::hessian_vector_ws_bytes(ld, nI, N, batch) : 0;
+        case OO_WS_HESSIAN_DIAGONAL: return oo::hessian_diagonal_ws_bytes(ld, nI);
         default: return 0;
     }
 }

@@ -129,6 +129,16 @@ class MOIntegrals:
             return self.eng.class_hessian(self.cls, F, d1, d2, pair_l=pair_l, pair_r=pair_r)[0]
         return self.eng.hessian(self.h[0], self.g[0], F[0], d1, d2, pair_l=pair_l, pair_r=pair_r)
 
+    def hessian_vector(self, F, d1, d2, V):
+        if self.kind == "class":
+            return self.eng.class_hessian_vector(self.cls[0], F[0], d1, d2, V)
+        return self.eng.hessian_vector(self.h[0], self.g[0], F[0], d1, d2, V)
+
+    def hessian_diagonal(self, F, d1, d2):
+        if self.kind == "class":
+            return self.eng.class_hessian_diagonal(self.cls[0], F[0], d1, d2)
+        return self.eng.hessian_diagonal(self.h[0], self.g[0], F[0], d1, d2)
+
 
 class HotPathEngine:
     _tensor_engines = {}
@@ -666,6 +676,32 @@ class HotPathEngine:
                                                   flags, self.stream), "class_hessian")
         return H
 
+    def class_hessian_vector(self, cls, F, d1, d2, V, out=None):
+        """H V (nk, nv) of ONE evaluation, cls (rows, ld, ld), F (ld, ld), V (nk, nv) device tensors, without
+        forming H."""
+        nk, nv = V.shape
+        HV = out if out is not None else torch.empty(nk, nv, dtype=F64, device=self.device)
+        if nk == 0 or nv == 0:
+            return HV
+        nbytes = self.lib.oo_workspace_bytes(_lib.OO_WS_CLASS_HESSIAN_VECTOR, self.na, self.ld, self.nI, nv)
+        ws = self.workspace("hvp", nbytes)
+        self._check(self.lib.oo_class_hessian_vector_f64(_p(cls), _p(F), _p(d1), _p(d2), self.no, self.na, self.N,
+                                                         self.ld, self.nIp, _p(self.pair_l), _p(self.pair_r), nk,
+                                                         _p(V), nv, _p(HV), _p(ws), nbytes, self.stream),
+                    "class_hessian_vector")
+        return HV
+
+    def class_hessian_diagonal(self, cls, F, d1, d2):
+        """diag(H) (nk,) of ONE evaluation from its class buffer."""
+        diag = torch.empty(self.nk, dtype=F64, device=self.device)
+        if self.nk == 0:
+            return diag
+        self._check(self.lib.oo_class_hessian_diagonal_f64(_p(cls), _p(F), _p(d1), _p(d2), self.no, self.na, self.N,
+                                                           self.ld, self.nIp, _p(self.pair_l), _p(self.pair_r),
+                                                           self.nk, _p(diag), None, 0, self.stream),
+                    "class_hessian_diagonal")
+        return diag
+
     def pairs_quarter_one(self):
         """True when `oo_class_transform_sym_f64` sends two evaluations of a batch through one quarter-1 GEMM (the
         same conditions as in csrc/classes.cu: 8-fold packed integrals shared by the batch, triangular quarter 2, a
@@ -760,6 +796,31 @@ class HotPathEngine:
                                             self.ld, _p(pl), _p(pr), nk, _p(H), _p(ws),
                                             nbytes, self.flags, self.stream), "hessian")
         return H
+
+    def hessian_vector(self, h, g, F, d1, d2, V, out=None):
+        """H V (nk, nv) of ONE evaluation from the complete transformed integrals (single padded h, g, F)."""
+        nk, nv = V.shape
+        HV = out if out is not None else torch.empty(nk, nv, dtype=F64, device=self.device)
+        if nk == 0 or nv == 0:
+            return HV
+        nbytes = self.lib.oo_workspace_bytes(_lib.OO_WS_HESSIAN_VECTOR, self.na, self.ld, self.nI, nv)
+        ws = self.workspace("hvp_full", nbytes)
+        self._check(self.lib.oo_hessian_vector_f64(_p(h), _p(g), _p(F), _p(d1), _p(d2), self.no, self.na, self.N,
+                                                   self.ld, _p(self.pair_l), _p(self.pair_r), nk, _p(V), nv, _p(HV),
+                                                   _p(ws), nbytes, self.stream), "hessian_vector")
+        return HV
+
+    def hessian_diagonal(self, h, g, F, d1, d2):
+        """diag(H) (nk,) of ONE evaluation from the complete transformed integrals."""
+        diag = torch.empty(self.nk, dtype=F64, device=self.device)
+        if self.nk == 0:
+            return diag
+        nbytes = self.lib.oo_workspace_bytes(_lib.OO_WS_HESSIAN_DIAGONAL, self.N, self.ld, self.nI, 1)
+        ws = self.workspace("hdiag_full", nbytes)
+        self._check(self.lib.oo_hessian_diagonal_f64(_p(h), _p(g), _p(F), _p(d1), _p(d2), self.no, self.na, self.N,
+                                                     self.ld, _p(self.pair_l), _p(self.pair_r), self.nk, _p(diag),
+                                                     _p(ws), nbytes, self.stream), "hessian_diagonal")
+        return diag
 
     def full_rdms(self, d1, d2):
         """Dense full-space RDMs (reference full_rdms, oo_energy.py:342-379): (N,N), (N,N,N,N)."""

@@ -218,7 +218,7 @@ class OrbitalHessian:
 
     def __init__(self, eng, ints, F, one_rdm, two_rdm, like):
         self._eng, self._ints, self._F = eng, ints, F
-        self._hold = ints.hold()                     # matrix() / dense() read the integrals later
+        self._hold = ints.hold()                     # matrix() / dense() / matvec() / diagonal() read the integrals later
         self._d1, self._d2 = eng.dev(one_rdm), eng.dev(two_rdm)
         self._like = like
         self.shape = (eng.N,) * 4
@@ -226,6 +226,24 @@ class OrbitalHessian:
     def matrix(self, pair_l=None, pair_r=None):
         """``H[l_j, r_j, l_k, r_k]`` for the engine's non-redundant pairs (or the given ones)."""
         return self._ints.hessian(self._F, self._d1, self._d2, pair_l=pair_l, pair_r=pair_r)
+
+    def matvec(self, v):
+        """``H @ v`` for ``v (n_kappa,)`` or ``(n_kappa, nv)`` (numpy or torch, any device), without forming H:
+        one streamed pass over the transformed integrals per block of vectors.  Same shape, array type and device
+        as ``v``."""
+        eng = self._eng
+        shape = tuple(v.shape)
+        if len(shape) not in (1, 2) or shape[0] != eng.nk:
+            raise ValueError(f"matvec expects ({eng.nk},) or ({eng.nk}, nv), got {shape}")
+        V = eng.dev(v).reshape(eng.nk, 1 if len(shape) == 1 else shape[1])
+        if V.numel() == 0:
+            return _like(torch.zeros(shape, dtype=F64, device=eng.device), v)
+        HV = self._ints.hessian_vector(self._F, self._d1, self._d2, V)
+        return _like(HV.reshape(shape), v)
+
+    def diagonal(self):
+        """``matrix().diagonal()`` without forming H, ``(n_kappa,)`` in the array type of ``full_hessian_to_matrix``."""
+        return _like(self._ints.hessian_diagonal(self._F, self._d1, self._d2), self._like)
 
     def dense(self):
         """The reference's rank-4 tensor ``H[p,q,r,s]`` (``oo_energy.py:311-340``); O(N^4) memory."""

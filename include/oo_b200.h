@@ -54,7 +54,11 @@ enum {
     OO_WS_CLASS_TRANSFORM = 6, /* oo_class_transform_f64 (nI = no+na)              */
     OO_WS_CLASS_BUFFER    = 7, /* size of the class buffer `cls` (x batch)         */
     OO_WS_CLASS_HESSIAN   = 8, /* oo_class_hessian_f64: pass N = na (!), nI = no+na, batch */
-    OO_WS_CLASS_TRANSFORM_SYM = 9 /* oo_class_transform_sym_f64 (nI = no+na)       */
+    OO_WS_CLASS_TRANSFORM_SYM = 9, /* oo_class_transform_sym_f64 (nI = no+na)      */
+    OO_WS_CLASS_HESSIAN_VECTOR = 10, /* oo_class_hessian_vector_f64: pass N = na (!), nI = no+na, batch = nv */
+    OO_WS_HESSIAN_VECTOR  = 11, /* oo_hessian_vector_f64: pass N = na (!), nI = no+na, batch = nv   */
+    OO_WS_HESSIAN_DIAGONAL = 12 /* oo_hessian_diagonal_f64 (nI = no+na); oo_class_hessian_diagonal_f64
+                                   needs no workspace                                              */
 };
 
 int         oo_abi_version(void);
@@ -297,6 +301,35 @@ int oo_class_hessian_f64(const double *cls, const double *F, const double *gamma
                          int nIp, int batch, const int32_t *pair_l, const int32_t *pair_r, int nk,
                          double *H, void *ws, size_t ws_bytes, unsigned flags, void *stream);
                          /* batched: cls[b], F[b] (ld^2), H[b] (nk^2) contiguous per evaluation */
+
+/* ---- K4, matrix free: Hessian-vector products and the Hessian diagonal ------------------------------------
+ * The same H as oo_class_hessian_f64 / oo_hessian_f64 (oo_energy.py:311-340, :342-379, :381-393, :395-402) for
+ * ONE evaluation, without forming it or the T-matrix.  V and HV are nk x nv, row-major: HV = H V.  With V the
+ * skew matrix of a vector (V[l_j, r_j] = v_j = -V[r_j, l_j]),
+ *   W[p,q] = -((F + F^T) V)[p,q] + [p in I] sum_{r in I, s} T[(p r),(q s)] V[r,s],   (H v)_j = W[l_j,r_j] - W[r_j,l_j],
+ * and the T part is one streamed pass over the class planes per block of up to 8 vectors (DMMA on each plane times
+ * the rows of At V it meets); larger nv is processed in blocks.  diag[j] = H[j][j] is a dot product of four
+ * columns of At with the class planes.  Every reduction runs in a fixed order: identical calls give identical
+ * bits.  Every unordered pair (pair_l[j], pair_r[j]) must occur at most once, pair_l[j] != pair_r[j].
+ * ws: oo_workspace_bytes(OO_WS_CLASS_HESSIAN_VECTOR, na, ld, no+na, nv) (pass N = na); the class diagonal needs
+ * no workspace (ws may be NULL).  The (h_mo, g_mo) forms first gather the class layout out of the complete g'
+ * into their workspace (OO_WS_HESSIAN_VECTOR with N = na and batch = nv, OO_WS_HESSIAN_DIAGONAL).             */
+int oo_class_hessian_vector_f64(const double *cls, const double *F, const double *gamma, const double *Gamma,
+                                int no, int na, int N, int ld, int nIp, const int32_t *pair_l,
+                                const int32_t *pair_r, int nk, const double *V, int nv, double *HV,
+                                void *ws, size_t ws_bytes, void *stream);
+int oo_class_hessian_diagonal_f64(const double *cls, const double *F, const double *gamma, const double *Gamma,
+                                  int no, int na, int N, int ld, int nIp, const int32_t *pair_l,
+                                  const int32_t *pair_r, int nk, double *diag, void *ws, size_t ws_bytes,
+                                  void *stream);
+int oo_hessian_vector_f64(const double *h_mo, const double *g_mo, const double *F, const double *gamma,
+                          const double *Gamma, int no, int na, int N, int ld, const int32_t *pair_l,
+                          const int32_t *pair_r, int nk, const double *V, int nv, double *HV,
+                          void *ws, size_t ws_bytes, void *stream);
+int oo_hessian_diagonal_f64(const double *h_mo, const double *g_mo, const double *F, const double *gamma,
+                            const double *Gamma, int no, int na, int N, int ld, const int32_t *pair_l,
+                            const int32_t *pair_r, int nk, double *diag, void *ws, size_t ws_bytes,
+                            void *stream);
 
 /* Lower triangle (diagonal included) of `batch` symmetric n x n matrices, rows back to back in np.tril_indices(n)
  * order: packed[b][i(i+1)/2 + j] = H[b][i][j], j <= i.  The orbital Hessian of full_hessian_to_matrix
