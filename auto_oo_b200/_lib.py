@@ -21,7 +21,7 @@ _u32 = C.c_uint
 
 OO_WS_ROTATION, OO_WS_INT2E, OO_WS_HESSIAN, OO_WS_INT1E, OO_WS_YMATRIX = 1, 2, 3, 4, 5
 OO_WS_CLASS_TRANSFORM, OO_WS_CLASS_BUFFER, OO_WS_CLASS_HESSIAN, OO_WS_CLASS_TRANSFORM_SYM = 6, 7, 8, 9
-OO_WS_CLASS_HESSIAN_VECTOR, OO_WS_HESSIAN_VECTOR, OO_WS_HESSIAN_DIAGONAL = 10, 11, 12
+OO_WS_CLASS_HESSIAN_VECTOR, OO_WS_HESSIAN_VECTOR, OO_WS_HESSIAN_DIAGONAL, OO_WS_KRYLOV = 10, 11, 12, 13
 # per-call variant switches (include/oo_b200.h)
 OO_FLAG_HESSIAN_DENSE, OO_FLAG_HESSIAN_ASSEMBLE_PER_ELEMENT, OO_FLAG_HESSIAN_ASSEMBLE_TILED = 1, 2, 4
 OO_FLAG_CLASS_UNFUSED_PACK, OO_FLAG_HESSIAN_GROUP_UNSTREAMED, OO_FLAG_HESSIAN_ASSEMBLE_UNSTREAMED = 8, 16, 32
@@ -90,6 +90,12 @@ _SIGNATURES = {
                                      _i32, _ptr, _ptr, _size, _ptr]),
     "oo_hessian_diagonal_f64": (_i32, [_ptr, _ptr, _ptr, _ptr, _ptr, _i32, _i32, _i32, _i32, _ptr, _ptr, _i32, _ptr,
                                        _ptr, _size, _ptr]),
+    "oo_subspace_eigh_f64": (_i32, [_ptr, _i32, _i32, _i64, _i32, _ptr, _i64, _ptr, _i32, _i64, _ptr]),
+    "oo_davidson_project_f64": (_i32, [_ptr, _i64, _i64, _i32, _ptr, _ptr, _i32, _ptr, _i32, _ptr]),
+    "oo_davidson_expand_f64": (_i32, [_ptr, _ptr, _i64, _i64, _i32, _i32, _ptr, _i32, _ptr, _ptr, _f64, _ptr, _i32,
+                                      _ptr, _ptr, _ptr, _ptr, _ptr, _size, _ptr]),
+    "oo_pcg_step_f64": (_i32, [_i64, _ptr, _f64, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _i32, _ptr, _size,
+                               _ptr]),
     "oo_pack_lower_f64": (_i32, [_ptr, _i32, _i32, _ptr, _ptr]),
     "oo_copy_f64": (_i32, [_ptr, _ptr, _i64, _ptr]),
     "oo_rdm_columns": (_i64, [_i32]),

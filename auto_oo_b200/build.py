@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB_PATH = os.path.join(OUT_DIR, "liboo_b200.so")
-SOURCES = ["api.cu", "dgemm_tn.cu", "dgemm_tri.cu", "dgemm_small.cu", "expm.cu", "contract.cu", "hessian.cu", "classes.cu", "rdm.cu"]
+SOURCES = ["api.cu", "dgemm_tn.cu", "dgemm_tri.cu", "dgemm_small.cu", "expm.cu", "contract.cu", "hessian.cu", "classes.cu", "rdm.cu", "krylov.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"),
            os.path.join(os.path.dirname(HERE), "include", "oo_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -23,6 +23,7 @@ size_t class_hessian_ws_bytes(int ld, int nIp, int no, int na, int batch);
 size_t class_hessian_vector_ws_bytes(int ld, int nIp, int no, int na, int nv);
 size_t hessian_vector_ws_bytes(int ld, int nI, int na, int nv);
 size_t hessian_diagonal_ws_bytes(int ld, int nI);
+size_t krylov_ws_bytes(int64_t n, int k);
 
 int sm_count() {
     static int cached[64] = {};                         // per device
@@ -169,6 +170,7 @@ size_t oo_workspace_bytes(int which, int N, int ld, int nI, int batch) {
         case OO_WS_HESSIAN_VECTOR:
             return (N > 0 && N <= nI) ? oo::hessian_vector_ws_bytes(ld, nI, N, batch) : 0;
         case OO_WS_HESSIAN_DIAGONAL: return oo::hessian_diagonal_ws_bytes(ld, nI);
+        case OO_WS_KRYLOV: return oo::krylov_ws_bytes(N, nI);   /* N carries the vector length, nI the basis size */
         default: return 0;
     }
 }

@@ -822,6 +822,42 @@ class HotPathEngine:
                                                      _p(ws), nbytes, self.stream), "hessian_diagonal")
         return diag
 
+    # ------------------------------------------------------------------ Krylov arithmetic between products (krylov.cu)
+    def krylov_workspace(self, n, kmax):
+        nbytes = self.lib.oo_workspace_bytes(_lib.OO_WS_KRYLOV, int(n), 1, int(kmax), 1)
+        return self.workspace("krylov", nbytes), nbytes
+
+    def subspace_eigh(self, S, k, w, Y):
+        """Ascending eigenvalues ``w[:k]`` and eigenvectors (columns of ``Y[:k, :k]``) of the leading k x k block of
+        the symmetric ``S`` (lower triangle read); ``S (m, m)`` or a batch ``(B, m, m)`` with ``w (B, m)``,
+        ``Y (B, m, m)``."""
+        B = S.shape[0] if S.dim() == 3 else 1
+        self._check(self.lib.oo_subspace_eigh_f64(_p(S), int(k), S.shape[-1], S.shape[-1] * S.shape[-2], B, _p(w),
+                                                  w.shape[-1], _p(Y), Y.shape[-1], Y.shape[-1] * Y.shape[-2],
+                                                  self.stream), "subspace_eigh")
+
+    def davidson_project(self, Vt, k, u, out, inc, out2=None, inc2=0):
+        """``out[j*inc] = Vt[j] . u`` (and ``out2[j*inc2]``) for j < k."""
+        self._check(self.lib.oo_davidson_project_f64(_p(Vt), Vt.shape[1], u.numel(), int(k), _p(u), _p(out), int(inc),
+                                                     _p(out2), int(inc2), self.stream), "davidson_project")
+
+    def davidson_expand(self, Vt, HVt, k, Y, theta, D, S, x, hx, yprev, rnorm, floor):
+        """Ritz pair of column 0 of Y, residual norm, and the next basis row (restart when k = rows of Vt)."""
+        n, kmax = D.numel(), Vt.shape[0]
+        ws, nbytes = self.krylov_workspace(n, kmax)
+        self._check(self.lib.oo_davidson_expand_f64(_p(Vt), _p(HVt), n, Vt.shape[1], int(k), kmax, _p(Y), Y.shape[1],
+                                                    _p(theta), _p(D), float(floor), _p(S), S.shape[1], _p(x), _p(hx),
+                                                    _p(yprev), _p(rnorm), _p(ws), nbytes, self.stream),
+                    "davidson_expand")
+
+    def pcg_step(self, Ap, shift, D, x, r, p, state, rnorm, w=None, aw=None, init=False):
+        """One deflated PCG step on (H + shift) x = b (``init``: the start from r = b); ``Ap = H p``."""
+        n = D.numel()
+        ws, nbytes = self.krylov_workspace(n, 1)
+        self._check(self.lib.oo_pcg_step_f64(n, _p(Ap), float(shift), _p(D), _p(w), _p(aw), _p(x), _p(r), _p(p),
+                                             _p(state), _p(rnorm), int(bool(init)), _p(ws), nbytes, self.stream),
+                    "pcg_step")
+
     def full_rdms(self, d1, d2):
         """Dense full-space RDMs (reference full_rdms, oo_energy.py:342-379): (N,N), (N,N,N,N)."""
         N = self.N
@@ -853,7 +889,7 @@ class HotPathEngine:
 
     # ------------------------------------------------------------------ whole evaluations
     def evaluate(self, oao_mo_coeff, d1, d2, kappa=None, want_hessian=True, squarings=None,
-                 H_out=None, stage_events=None, path="class", on_result=None):
+                 H_out=None, stage_events=None, path="class", on_result=None, on_integrals=None):
         """E (B,), packed gradient (B, nk) and Hessian (B, nk, nk) at C' = X C_oao expm(-K(kappa_b)).
 
         ``oao_mo_coeff``: padded (ld, ld) or (B, ld, ld) device tensor; ``kappa``: (B, nk) or None.
@@ -866,7 +902,10 @@ class HotPathEngine:
         "fock_gradient", "hessian"), a list of (start, end) CUDA-event pairs recorded on the launching stream
         around the kernels of that stage (bench.py's roofline figures).
         ``on_result(b)`` is called after the kernels of evaluation ``b`` are enqueued (used to start
-        the device->host copy of its Hessian while evaluation ``b+1`` computes)."""
+        the device->host copy of its Hessian while evaluation ``b+1`` computes).
+        ``on_integrals(b, ints, F, g)`` is called with the :class:`MOIntegrals` of evaluation ``b``, its generalized
+        Fock matrix ``F (1, ld, ld)`` and its gradient ``g (nk,)`` while they are valid: the next evaluation of the
+        call reuses their buffer."""
         def staged(name, fn):
             if stage_events is None:
                 return fn()
@@ -910,6 +949,10 @@ class HotPathEngine:
                 G[lo:hi] = gv
                 if want_hessian:
                     staged("hessian", lambda: self.class_hessian(cbuf, F, d1b, d2b, out=H[lo:hi]))
+                if on_integrals is not None:
+                    for b in range(lo, hi):
+                        on_integrals(b, MOIntegrals(self, "class", cls=cbuf[b - lo:b - lo + 1]), F[b - lo:b - lo + 1],
+                                     gv[b - lo])
                 if on_result is not None:
                     for b in range(lo, hi):
                         on_result(b)
@@ -928,6 +971,8 @@ class HotPathEngine:
             G[b] = gv[0]
             if want_hessian:
                 self.hessian(h1[0], gbuf[0], F[0], d1b, d2b, out=H[b])
+            if on_integrals is not None:
+                on_integrals(b, MOIntegrals(self, "full", h=h1, g=gbuf), F, gv[0])
             if on_result is not None:
                 on_result(b)
         self._park("full", gbuf)

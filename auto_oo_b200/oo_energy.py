@@ -245,6 +245,52 @@ class OrbitalHessian:
         """``matrix().diagonal()`` without forming H, ``(n_kappa,)`` in the array type of ``full_hessian_to_matrix``."""
         return _like(self._ints.hessian_diagonal(self._F, self._d1, self._d2), self._like)
 
+    # ---- matrix-free second-order steps (auto_oo_b200/krylov.py): products and the diagonal only, H never formed
+    def _device_matvec(self, v):
+        shape = tuple(v.shape)
+        V = v.reshape(self._eng.nk, -1).contiguous()
+        return self._ints.hessian_vector(self._F, self._d1, self._d2, V).reshape(shape)
+
+    def _device_diagonal(self):
+        return self._ints.hessian_diagonal(self._F, self._d1, self._d2)
+
+    def lowest_eigenpair(self, tol=1e-7, max_iter=200, info=None):
+        """``(lambda_0, x_0)``: the lowest eigenvalue of H and its unit eigenvector (in the array type of
+        :meth:`diagonal`) by Davidson on :meth:`matvec`, to ``||H x_0 - lambda_0 x_0|| <= tol``.  A negative
+        ``lambda_0`` at a converged orbital optimisation means a saddle point, not a minimum."""
+        from . import krylov
+        if self._eng.nk == 0:
+            raise ValueError("the Hessian has no parameters")
+        lam, x = krylov.lowest_eigenpair(self._device_matvec, self._device_diagonal(), tol=tol, max_iter=max_iter,
+                                         engine=self._eng, info=info)
+        return lam, _like(x, self._like)
+
+    def solve(self, rhs, shift=0.0, tol=1e-12, max_iter=1000, info=None):
+        """``(H + shift)^-1 rhs`` by preconditioned CG on :meth:`matvec` (``H + shift`` must be positive definite),
+        to ``||(H + shift) x - rhs|| <= tol ||rhs||``; same array type, device and shape as ``rhs (n_kappa,)``."""
+        from . import krylov
+        nk = self._eng.nk
+        if tuple(rhs.shape) != (nk,):
+            raise ValueError(f"solve expects ({nk},), got {tuple(rhs.shape)}")
+        x = krylov.shifted_solve(self._device_matvec, self._device_diagonal(), self._eng.dev(rhs), shift=shift,
+                                 tol=tol, max_iter=max_iter, engine=self._eng, info=info)
+        return _like(x, rhs)
+
+    def newton_step(self, gradient, mu=1e-6, rho=1.1, lambda_min=1e-6, aug=True, eig_tol=1e-7, lin_tol=1e-12,
+                    eig_max_iter=200, lin_max_iter=1000, info=None):
+        """``(dp, lambda_0)`` of ``NewtonStep.newton_step(gradient, matrix())`` without forming H: Davidson for the
+        lowest eigenpair, deflated PCG for ``dp = -(H + sigma)^-1 g``.  ``dp`` has the array type, device and shape of
+        ``gradient (n_kappa,)``.  ``aug=False`` with ``lambda_0 < lambda_min`` raises ``ValueError`` (indefinite
+        system: use the formed matrix); no convergence raises ``RuntimeError``."""
+        from . import krylov
+        nk = self._eng.nk
+        if tuple(gradient.shape) != (nk,):
+            raise ValueError(f"newton_step expects a gradient of shape ({nk},), got {tuple(gradient.shape)}")
+        dp, lam = krylov.newton_step(self._device_matvec, self._device_diagonal(), self._eng.dev(gradient), mu=mu,
+                                     rho=rho, lambda_min=lambda_min, aug=aug, eig_tol=eig_tol, lin_tol=lin_tol,
+                                     eig_max_iter=eig_max_iter, lin_max_iter=lin_max_iter, engine=self._eng, info=info)
+        return _like(dp, gradient), lam
+
     def dense(self):
         """The reference's rank-4 tensor ``H[p,q,r,s]`` (``oo_energy.py:311-340``); O(N^4) memory."""
         N = self._eng.N
@@ -597,12 +643,15 @@ class OO_energy:
                                     copy=not pinned_results)
         return pending.wait() if wait else pending
 
-    def energy_gradient_newton_direction(self, kappa, one_rdm, two_rdm, **newton_kwargs):
+    def energy_gradient_newton_direction(self, kappa, one_rdm, two_rdm, matrix_free=False, **newton_kwargs):
         """Device-resident Newton mode of :meth:`energy_gradient_hessian`: for every rotation of the batch the
         Hessian is built AND consumed in HBM -- ``NewtonStep.newton_step`` (one ``eigh`` on the device, the
         augmented-Hessian shift of ``utils/newton_raphson.py:78-129``) -- and only ``E (B,)``, the gradient
         ``(B, n_kappa)``, the Newton direction ``(B, n_kappa)`` and the lowest Hessian eigenvalue ``(B,)`` come
-        back (on the device of ``kappa``).  ``newton_kwargs`` go to :class:`NewtonStep` (``mu, rho, lambda_min, aug``)."""
+        back (on the device of ``kappa``).  ``newton_kwargs`` go to :class:`NewtonStep` (``mu, rho, lambda_min, aug``).
+        ``matrix_free=True``: each rotation evaluates E and G only, and the step comes from an :class:`OrbitalHessian`
+        on that rotation's transformed integrals (Davidson + deflated CG on products, ``OrbitalHessian.newton_step``):
+        H is never formed, E and G are the same, the direction and eigenvalue agree to the solver tolerances."""
         eng = self.engine
         kappa = _as_tensor(kappa).detach().reshape(-1, self.n_kappa)
         dev_in = kappa.device
@@ -613,6 +662,17 @@ class OO_energy:
         dk = torch.empty(B, self.n_kappa, dtype=F64, device=eng.device)
         lam = torch.empty(B, dtype=F64)
         Es, Gs = [], []
+        if matrix_free:
+            for b in range(B):
+                d1b, d2b = d1[b:b + 1] if d1.dim() == 3 else d1, d2[b:b + 1] if d2.dim() == 5 else d2
+
+                def step(_, ints, F, g):                         # while this rotation's integrals are current
+                    dk[b], lam[b] = opt.newton_step(g, OrbitalHessian(eng, ints, F, d1b, d2b, d1b))
+                E, G, _ = eng.evaluate(Coao, d1b, d2b, kappa=kd[b:b + 1], want_hessian=False, path=self.integral_path,
+                                       on_integrals=step)
+                Es.append(E)
+                Gs.append(G)
+            return (torch.cat(Es).to(dev_in), torch.cat(Gs).to(dev_in), dk.to(dev_in), lam.to(dev_in))
         H = eng.workspace_tensor("H_newton", (1, self.n_kappa, self.n_kappa))
         for b in range(B):                                   # one Hessian resident at a time
             E, G, _ = eng.evaluate(Coao, d1[b:b + 1] if d1.dim() == 3 else d1, d2[b:b + 1] if d2.dim() == 5 else d2,
@@ -624,10 +684,13 @@ class OO_energy:
 
     # ------------------------------------------------------------------ driver
     def orbital_optimization(self, one_rdm, two_rdm, conv_tol=1e-8, max_iterations=100, verbose=0,
-                             **kwargs):
+                             matrix_free=False, **kwargs):
         """Damped-Newton orbital optimisation at fixed RDMs; mutates ``oao_mo_coeff`` and returns
         the energy trajectory (reference ``oo_energy.py:426-474``: re-base after every step,
-        convergence tested only for ``n > 1``, per-iteration line printed unless ``verbose`` is None)."""
+        convergence tested only for ``n > 1``, per-iteration line printed unless ``verbose`` is None).
+        ``matrix_free=True``: every iteration takes the gradient and the :class:`OrbitalHessian` at the current
+        orbitals (one transform, shared through the integral cache) and ``NewtonStep`` steps on its products; the
+        n_kappa^2 Hessian is never formed.  The trajectory equals the default one to the solver tolerances."""
         objective_fn = partial(self.energy_from_kappa, one_rdm=one_rdm, two_rdm=two_rdm)
         # batched form for NewtonStep(speculate=k): a list of (kappa,) tuples -> energies
         objective_fn.batched = lambda plist: self.energies_from_kappas(
@@ -642,9 +705,19 @@ class OO_energy:
             kappa = torch.zeros(self.n_kappa, dtype=F64, device=one.device)
             # gradient and Hessian at the current orbitals from ONE fused evaluation (one transform, one graph
             # replay for small bases) instead of the reference's analytic_gradient + analytic_hessian calls
-            _, G, H = self.energy_gradient_hessian(kappa[None], one_rdm, two_rdm)
-            gradient, hessian = G[0], H[0]
-            kappa, lowest_eigenvalue = opt.damped_newton_step(objective_fn, (kappa,), gradient, hessian)
+            if matrix_free:
+                ints = self._mo_integrals()
+                d1, d2 = self.engine.dev(one_rdm), self.engine.dev(two_rdm)
+                _, _, F, _, gv = ints.fock_gradient(d1, d2, want_matrix=False)
+                gradient = gv[0].to(one.device)
+                # damped_newton_step in two parts: the OrbitalHessian (and its hold on the integrals) is released
+                # before the line search, whose transforms then reuse the cached class buffer
+                dp, lowest_eigenvalue = opt.newton_step(gradient, OrbitalHessian(self.engine, ints, F, d1, d2, d1))
+                kappa, _ = opt.backtracking(objective_fn, (kappa,), dp, gradient)
+            else:
+                _, G, H = self.energy_gradient_hessian(kappa[None], one_rdm, two_rdm)
+                gradient, hessian = G[0], H[0]
+                kappa, lowest_eigenvalue = opt.damped_newton_step(objective_fn, (kappa,), gradient, hessian)
             self.oao_mo_coeff = self.get_transformed_mo(self.oao_mo_coeff, kappa)
             energy = self.energy_from_mo_coeff(self.mo_coeff, one_rdm, two_rdm).item()
             energy_l.append(energy)

@@ -40,7 +40,11 @@ class NewtonStep:
         self.speculate = int(speculate)
 
     def newton_step(self, gradient, hessian):
-        """Returns ``(dp, lowest eigenvalue of the un-augmented Hessian)`` (reference ``:78-129``)."""
+        """Returns ``(dp, lowest eigenvalue of the un-augmented Hessian)`` (reference ``:78-129``).  ``hessian`` is a
+        matrix, or an operator with ``matvec`` and ``diagonal`` (``OrbitalHessian``): then H is never formed -- Davidson
+        finds the lowest eigenpair and deflated CG solves the shifted system (``auto_oo_b200/krylov.py``)."""
+        if hasattr(hessian, "matvec") and hasattr(hessian, "diagonal"):
+            return self._matrix_free_step(gradient, hessian)
         evals, evecs = torch.linalg.eigh(hessian)
         lowest_eigenvalue = evals[0].item()
         if self.verbose:
@@ -55,6 +59,20 @@ class NewtonStep:
                 print("Lowest eigenvalue of augmented hessian:", evals[0].item())
         # -(V diag(1/w) V^T) g without forming the inverse
         return -(evecs @ ((evecs.T @ gradient) / evals)), lowest_eigenvalue
+
+    def _matrix_free_step(self, gradient, hessian):
+        kw = dict(mu=self.mu, rho=self.rho, lambda_min=self.lambda_min, aug=self.aug)
+        if hasattr(hessian, "newton_step"):
+            dp, lowest_eigenvalue = hessian.newton_step(gradient, **kw)
+        else:
+            from .. import krylov
+            dp, lowest_eigenvalue = krylov.newton_step(hessian.matvec, hessian.diagonal(), gradient, **kw)
+            dp = dp.to(gradient.device)
+        if self.verbose:
+            print("lowest eigval hessian =", lowest_eigenvalue)
+            if lowest_eigenvalue < self.lambda_min and self.aug:
+                print("augmenting hessian...")
+        return dp, lowest_eigenvalue
 
     def backtracking(self, objective_fn, parameters, dp, gradient):
         """Reference ``:131-192``."""

@@ -57,8 +57,10 @@ enum {
     OO_WS_CLASS_TRANSFORM_SYM = 9, /* oo_class_transform_sym_f64 (nI = no+na)      */
     OO_WS_CLASS_HESSIAN_VECTOR = 10, /* oo_class_hessian_vector_f64: pass N = na (!), nI = no+na, batch = nv */
     OO_WS_HESSIAN_VECTOR  = 11, /* oo_hessian_vector_f64: pass N = na (!), nI = no+na, batch = nv   */
-    OO_WS_HESSIAN_DIAGONAL = 12 /* oo_hessian_diagonal_f64 (nI = no+na); oo_class_hessian_diagonal_f64
+    OO_WS_HESSIAN_DIAGONAL = 12, /* oo_hessian_diagonal_f64 (nI = no+na); oo_class_hessian_diagonal_f64
                                    needs no workspace                                              */
+    OO_WS_KRYLOV = 13          /* oo_davidson_expand_f64 / oo_pcg_step_f64: pass N = n (vector length), nI = k
+                                  (largest basis, <= 64), ld = batch = 1                                        */
 };
 
 int         oo_abi_version(void);
@@ -330,6 +332,45 @@ int oo_hessian_diagonal_f64(const double *h_mo, const double *g_mo, const double
                             const double *Gamma, int no, int na, int N, int ld, const int32_t *pair_l,
                             const int32_t *pair_r, int nk, double *diag, void *ws, size_t ws_bytes,
                             void *stream);
+
+/* ---- Krylov arithmetic between products: lowest Hessian eigenpair (Davidson-Liu) and shifted Newton solve (PCG) ----
+ * The products themselves are oo_class_hessian_vector_f64 / oo_hessian_vector_f64; these entry points are the solver
+ * arithmetic between them (auto_oo_b200/krylov.py drives them).  Vectors have length n; a Davidson basis is stored
+ * as ROWS Vt[j][0..n) (row pitch ldv), with its products HVt[j] = H Vt[j].  Every reduction runs in a fixed order
+ * (per-CTA block sums, then the CTA partials in CTA order): identical calls give identical bits; no host sync.
+ *
+ *  oo_subspace_eigh_f64     eigenvalues (ascending) w[b][0..k) and eigenvectors Y[b] (column j of the k x k
+ *                           row-major Y, pitch ldy, belongs to w[j]) of `batch` symmetric k x k matrices S[b] (pitch
+ *                           lds; the lower triangle is read), k <= 64: one CTA per matrix, cyclic Jacobi in shared
+ *                           memory.
+ *  oo_davidson_project_f64  out[j*inc] = Vt[j] . u for j < k (and out2[j*inc2] when out2 != NULL): the new row and
+ *                           column of S = V^T H V after the product u = H Vt[m].
+ *  oo_davidson_expand_f64   with y = column 0 of Y and theta = *theta (device): x = V^T y, hx = HV^T y,
+ *                           r = hx - theta x, *rnorm = ||r||, t = r / (D - theta) with |D - theta| floored at `floor_`,
+ *                           two-pass classical Gram-Schmidt of t against the basis, t / ||t|| -> Vt[k].  When k == kmax
+ *                           the basis restarts first: Vt[0] = x, Vt[1] = the previous Ritz vector (yprev, kept by the
+ *                           previous call) made orthonormal to x, HVt[0..1] and S[0..1][0..1] to match, t -> Vt[2].
+ *                           Vt, HVt need kmax rows, S is kmax x kmax (pitch lds), yprev kmax doubles (zero at first).
+ *                           rnorm[0] = ||r||; rnorm[1] = 1 when the orthogonalised correction vanished against the
+ *                           basis (breakdown: the new row is written as zeros), else 0.
+ *  oo_pcg_step_f64          deflated preconditioned CG on (H + shift) x = b with preconditioner D + shift (> 0) and the
+ *                           deflation vector w, aw = (H + shift) w (both NULL: plain PCG).  init != 0: r holds b on
+ *                           entry; x = w (w.b)/(w.aw), r = b - aw (w.b)/(w.aw), p = z - w (aw.z)/(w.aw), Ap unused.
+ *                           init == 0: Ap = H p (no shift): alpha = (r.z)/(p.(Ap + shift p)), x += alpha p,
+ *                           r -= alpha (Ap + shift p), z = r / (D + shift), p = z + beta p - w (aw.z)/(w.aw).
+ *                           state[0..1] carries r.z and w.aw between calls; *rnorm = ||r||.
+ * ws: oo_workspace_bytes(OO_WS_KRYLOV, n, 1, kmax, 1).  k > 64, null pointers and pitches below the length give
+ * OO_ERR_INVALID_ARG, a short workspace OO_ERR_WORKSPACE, both before any launch.                                 */
+int oo_subspace_eigh_f64(const double *S, int k, int lds, int64_t strideS, int batch, double *w, int64_t stridew,
+                         double *Y, int ldy, int64_t strideY, void *stream);
+int oo_davidson_project_f64(const double *Vt, int64_t ldv, int64_t n, int k, const double *u, double *out, int inc,
+                            double *out2, int inc2, void *stream);
+int oo_davidson_expand_f64(double *Vt, double *HVt, int64_t n, int64_t ldv, int k, int kmax, const double *Y, int ldy,
+                           const double *theta, const double *D, double floor_, double *S, int lds, double *x,
+                           double *hx, double *yprev, double *rnorm, void *ws, size_t ws_bytes, void *stream);
+int oo_pcg_step_f64(int64_t n, const double *Ap, double shift, const double *D, const double *w, const double *aw,
+                    double *x, double *r, double *p, double *state, double *rnorm, int init, void *ws, size_t ws_bytes,
+                    void *stream);
 
 /* Lower triangle (diagonal included) of `batch` symmetric n x n matrices, rows back to back in np.tril_indices(n)
  * order: packed[b][i(i+1)/2 + j] = H[b][i][j], j <= i.  The orbital Hessian of full_hessian_to_matrix
