@@ -885,6 +885,7 @@ hess_assemble_stream_kernel(TView tv, const double *__restrict__ F, const int32_
                 double v = q_in ? stage[((size_t)jj * S + sx) * kAsmRows + lane] : 0.0;
                 if (p_in) v -= __ldg(tv.row(p, sx, ld2) + (int64_t)q * ld + r);
                 if (q == sx) v -= fock_sym(F, ld, p, r);
+                if (q == r) v += fock_sym(F, ld, p, sx);      // (q >= rows_in: a pair (p, q) in a row inside I)
                 if (p == sx) v += fock_sym(F, ld, q, r);
                 if (p == r) v -= fock_sym(F, ld, q, sx);
                 strip[lane * (S + 1) + sx] = v;

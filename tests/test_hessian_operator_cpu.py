@@ -86,3 +86,59 @@ def test_plane_products_never_need_the_t_matrix(name):
         M = A[k] @ V[:ni]                                        # [p, s]
         streamed += M @ B[k].T                                   # [p, q] += sum_s M[p,s] B_k[q,s]
     assert (streamed - direct).abs().max().item() <= 1e-12 * max(1.0, direct.abs().max().item())
+
+
+# ---- the float64 reference of tests/test_gpu_hessian_configs.py, pinned ------------------------------------------------
+from test_gpu_hessian_configs import hessian_reference, low_rank_factors, t_reference  # noqa: E402
+
+
+@pytest.mark.parametrize("name", CASES)
+def test_generalised_reference_equals_the_class_oracle_on_tril_lists(name):
+    """T and H written out for an arbitrary pair list reproduce ClassEvaluation.hessian on the engine's list"""
+    c, ev = _evaluation(name)
+    one, two = c.one_rdm, c.two_rdm
+    T = t_reference(ev.h, ev.J, ev.K, one, two, ev.no, ev.na)
+    rr, cc = orc.tril_pairs(ev.N)
+    H = hessian_reference(T, ev.fock_generalized(one, two), ev.ni, rr[ev.params_idx], cc[ev.params_idx])
+    want = ev.hessian(one, two)
+    assert (H - want).abs().max().item() <= 1e-13 * want.abs().max().item()
+
+
+@pytest.mark.parametrize("name", ["n7_cas44", "n11_cas43"])
+def test_generalised_reference_reproduces_the_golden_hessians(name):
+    c, ev = _evaluation(name)
+    one, two = c.one_rdm, c.two_rdm
+    T = t_reference(ev.h, ev.J, ev.K, one, two, ev.no, ev.na)
+    rr, cc = orc.tril_pairs(ev.N)
+    H = hessian_reference(T, ev.fock_generalized(one, two), ev.ni, rr[ev.params_idx], cc[ev.params_idx])
+    assert np.abs(H.numpy() - c.ref["H"]).max() < 1e-12
+
+
+def test_generalised_reference_equals_the_dense_hessian_on_any_pair_list():
+    """upper-triangle, virt-virt and occ-occ pairs in random order: oo_oracle.hessian_full (dense N^4 / N^6) indexed
+    at the pairs"""
+    from auto_oo_b200.synthetic import random_rdms
+    N, no, na = 9, 2, 3
+    nI = no + na
+    M, w = low_rank_factors(N, N, seed=11)
+    g = torch.einsum('P,Pab,Pcd->abcd', w, M, M)
+    gen = torch.Generator().manual_seed(12)
+    h = torch.randn(N, N, dtype=DT, generator=gen)
+    h = h + h.T
+    one, two = random_rdms(na, 2, seed=3)
+    occ, act = np.arange(no), np.arange(no, nI)
+    H4 = orc.hessian_full(h, g, one, two, occ, act)
+    F = orc.fock_generalized(h, g, one, two, occ, act)
+    J = g[:, :, :nI, :nI].permute(2, 3, 0, 1)                   # J[m,n,a,b] = g'[a,b,m,n]
+    K = g[:, :nI, :nI, :].permute(2, 1, 0, 3)                   # K[n,m,a,b] = g'[a,m,n,b]
+    T = t_reference(h, J, K, one, two, no, na)
+    rng = np.random.default_rng(4)
+    rows, cols = np.tril_indices(N, k=-1)
+    flip = rng.random(len(rows)) < 0.5
+    L, R = np.where(flip, cols, rows), np.where(flip, rows, cols)
+    perm = rng.permutation(len(L))
+    L, R = L[perm], R[perm]
+    H = hessian_reference(T, F, nI, L, R)
+    Lt, Rt = torch.as_tensor(L), torch.as_tensor(R)
+    want = H4[Lt[:, None], Rt[:, None], Lt[None, :], Rt[None, :]]
+    assert (H - want).abs().max().item() <= 1e-13 * want.abs().max().item()
