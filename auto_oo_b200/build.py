@@ -7,6 +7,7 @@ on a machine without a GPU driver (nvcc cross-compiles; no GPU needed to build).
 """
 from __future__ import annotations
 
+import glob
 import hashlib
 import os
 import shutil
@@ -18,9 +19,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB_PATH = os.path.join(OUT_DIR, "liboo_b200.so")
-SOURCES = ["api.cu", "dgemm_tn.cu", "dgemm_tri.cu", "dgemm_small.cu", "expm.cu", "contract.cu", "hessian.cu", "classes.cu", "rdm.cu", "krylov.cu"]
-HEADERS = [os.path.join(CSRC, "common.cuh"),
-           os.path.join(os.path.dirname(HERE), "include", "oo_b200.h")]
+SOURCES = ["api.cu", "dgemm_tn.cu", "dgemm_tri.cu", "dgemm_small.cu", "expm.cu", "contract.cu", "hessian.cu",
+           "hessian_operator.cu", "classes.cu", "rdm.cu", "krylov.cu"]
+# every header a source may include: an edit to any of them rebuilds the library
+HEADERS = (sorted(glob.glob(os.path.join(CSRC, "*.cuh")))
+           + [os.path.join(os.path.dirname(HERE), "include", "oo_b200.h")])
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

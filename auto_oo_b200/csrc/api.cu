@@ -9,22 +9,6 @@ namespace oo {
 int g_last_cuda_error = 0;
 unsigned long long g_launch_count = 0;
 
-int dgemm_tn(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
-             int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
-             int64_t strideC, cudaStream_t stream);
-size_t rotation_ws_bytes(int ld, int batch);
-size_t int1e_ws_bytes(int ld, int batch);
-size_t hessian_ws_bytes(int ld, int nI);
-size_t y_matrix_ws_bytes(int ld, int N);
-size_t class_transform_ws_bytes(int ld, int nIp, int batch);
-size_t class_buffer_bytes(int ld, int nIp);
-size_t class_transform_sym_ws_bytes(int ld, int nIp, int batch);
-size_t class_hessian_ws_bytes(int ld, int nIp, int no, int na, int batch);
-size_t class_hessian_vector_ws_bytes(int ld, int nIp, int no, int na, int nv);
-size_t hessian_vector_ws_bytes(int ld, int nI, int na, int nv);
-size_t hessian_diagonal_ws_bytes(int ld, int nI);
-size_t krylov_ws_bytes(int64_t n, int k);
-
 int sm_count() {
     static int cached[64] = {};                         // per device
     int dev = 0, n = 0;

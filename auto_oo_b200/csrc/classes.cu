@@ -23,39 +23,6 @@
 
 namespace oo {
 
-int dgemm_tn(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
-             int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
-             int64_t strideC, cudaStream_t stream);
-int dgemm_tn_swap02(const double *At, const double *B, double *C, double *C2, int d0, int d1, int d2,
-                    int64_t N, int64_t K, int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA,
-                    int64_t strideB, int64_t strideC, cudaStream_t stream);
-int dgemm_tn_pair_unpack(const double *At, const double *B, double *C, double *C2, int d0, int dorb, int dP,
-                         int64_t N, int64_t K, int64_t lda, int64_t ldb, int64_t ldc, int batch,
-                         int64_t strideA, int64_t strideB, int64_t strideC, int64_t strideC2,
-                         cudaStream_t stream);
-
-int dgemm_tn_class_pack(const double *At, const double *B, double *P, int tri_rows, int nclass, int dorb,
-                        int64_t nrows2, int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int batch,
-                        int64_t strideA, int64_t strideB, int64_t strideP, cudaStream_t stream, int64_t r2_offset = 0);
-
-int dgemm_tn_q1_packed8(const double *A8, int64_t a8_ld, int pq_lo, int pq_cnt, const double *B, double *C,
-                        double *C2, int dorb, int dP, int64_t N, int64_t K, int64_t ldb, int64_t ldc, int batch,
-                        int64_t strideA8, int64_t strideB, int64_t strideC, int64_t strideC2, cudaStream_t stream,
-                        bool direct_epilogue);
-bool dgemm_tn_tri_supported(int nclass);
-int dgemm_tn_tri_class_pack(const double *At, const double *B, double *P, int tri_rows, int nclass, int dorb,
-                            int64_t ngroups, int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int batch,
-                            int64_t strideA, int64_t strideB, int64_t strideP, cudaStream_t stream,
-                            int64_t group_offset = 0, int64_t group_ld = 0, int halves = 1);
-
-int dgemm_tn_class_expand(const double *At, const double *B, double *Out, int transpose_mirror, int nclass, int dorb,
-                          int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int64_t ld_out, int batch,
-                          int64_t strideA, int64_t strideB, int64_t strideOut, cudaStream_t stream,
-                          bool direct_epilogue = false);
-int dgemm_tn_direct(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
-                    int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
-                    int64_t strideC, cudaStream_t stream);
-
 namespace {
 
 // dst[c][r] = src[r][c]  (rows x cols doubles), 32x32 tiles through padded shared memory

@@ -53,6 +53,11 @@ inline bool once_per_device(unsigned long long &mask) {
     return true;
 }
 
+// compile-time booleans for generic lambdas, e.g. a GEMM main loop's k-block body called with TrueTag{} for the last
+// k-block only
+struct FalseTag { static constexpr bool value = false; };
+struct TrueTag { static constexpr bool value = true; };
+
 // ---- FP64 tensor-core MMA (DMMA.8x8x4) --------------------------------------
 // Fragment ownership for lane = 4*g + t (g = 0..7, t = 0..3):
 //   a = A[g][t]   (row-major 8x4),  b = B[t][g]  (col-major 4x8),
@@ -192,5 +197,66 @@ struct ClassView {
 int encode_tmap_3d_f64(CUtensorMap *map, const void *base, uint64_t dim0, uint64_t dim1,
                        uint64_t dim2, uint64_t stride1_elems, uint64_t stride2_elems,
                        uint32_t box0, uint32_t box1);
+int encode_tmap_4d_f64(CUtensorMap *map, const void *base, const uint64_t dims[4], const uint64_t strides_elems[3],
+                       const uint32_t box[4]);
+
+// ---- host: functions one source file defines and others call ------------------
+// TN-GEMMs on the FP64 tensor pipe (dgemm_tn.cu, dgemm_tri.cu)
+int dgemm_tn(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
+             int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
+             int64_t strideC, cudaStream_t stream);
+int dgemm_tn_direct(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
+                    int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
+                    int64_t strideC, cudaStream_t stream);
+int dgemm_tn_swap02(const double *At, const double *B, double *C, double *C2, int d0, int d1, int d2,
+                    int64_t N, int64_t K, int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA,
+                    int64_t strideB, int64_t strideC, cudaStream_t stream);
+int dgemm_tn_pair_unpack(const double *At, const double *B, double *C, double *C2, int d0, int dorb, int dP,
+                         int64_t N, int64_t K, int64_t lda, int64_t ldb, int64_t ldc, int batch,
+                         int64_t strideA, int64_t strideB, int64_t strideC, int64_t strideC2,
+                         cudaStream_t stream);
+int dgemm_tn_class_pack(const double *At, const double *B, double *P, int tri_rows, int nclass, int dorb,
+                        int64_t nrows2, int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int batch,
+                        int64_t strideA, int64_t strideB, int64_t strideP, cudaStream_t stream, int64_t r2_offset = 0);
+int dgemm_tn_q1_packed8(const double *A8, int64_t a8_ld, int pq_lo, int pq_cnt, const double *B, double *C,
+                        double *C2, int dorb, int dP, int64_t N, int64_t K, int64_t ldb, int64_t ldc, int batch,
+                        int64_t strideA8, int64_t strideB, int64_t strideC, int64_t strideC2, cudaStream_t stream,
+                        bool direct_epilogue);
+int dgemm_tn_class_expand(const double *At, const double *B, double *Out, int transpose_mirror, int nclass, int dorb,
+                          int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int64_t ld_out, int batch,
+                          int64_t strideA, int64_t strideB, int64_t strideOut, cudaStream_t stream,
+                          bool direct_epilogue = false);
+bool dgemm_tn_tri_supported(int nclass);
+int dgemm_tn_tri_class_pack(const double *At, const double *B, double *P, int tri_rows, int nclass, int dorb,
+                            int64_t ngroups, int64_t npair_ld, int64_t K, int64_t lda, int64_t ldb, int batch,
+                            int64_t strideA, int64_t strideB, int64_t strideP, cudaStream_t stream,
+                            int64_t group_offset = 0, int64_t group_ld = 0, int halves = 1);
+// small GEMM on the FP64 tensor pipe (dgemm_small.cu)
+int dgemm_small(int transA, int transB, int M, int N, int K, double alpha, const double *A, int lda,
+                int64_t strideA, const double *B, int ldb, int64_t strideB, double beta,
+                const double *E, int lde, int64_t strideE, double gamma, double *D, int ldd,
+                int64_t strideD, int batch, cudaStream_t stream, int eye_n);
+
+// the class Hessian and the gathered class layout of the (h', g') forms (hessian.cu)
+int class_hessian(const double *cls, const double *F, const double *d1, int64_t sd1, const double *d2,
+                  int64_t sd2, int no, int na, int N, int ld, int nIp, int batch, const int32_t *pl,
+                  const int32_t *pr, int nk, double *H, void *ws, size_t ws_bytes, unsigned flags,
+                  cudaStream_t stream);
+int gather_class_layout(const double *h, const double *g, int nI, int ld, double *B, cudaStream_t stream);
+size_t full_hessian_b_bytes(int ld, int nIp);
+
+// workspace and buffer sizes (oo_workspace_bytes)
+size_t rotation_ws_bytes(int ld, int batch);
+size_t int1e_ws_bytes(int ld, int batch);
+size_t hessian_ws_bytes(int ld, int nI);
+size_t y_matrix_ws_bytes(int ld, int N);
+size_t class_transform_ws_bytes(int ld, int nIp, int batch);
+size_t class_buffer_bytes(int ld, int nIp);
+size_t class_transform_sym_ws_bytes(int ld, int nIp, int batch);
+size_t class_hessian_ws_bytes(int ld, int nIp, int no, int na, int batch);
+size_t class_hessian_vector_ws_bytes(int ld, int nIp, int no, int na, int nv);
+size_t hessian_vector_ws_bytes(int ld, int nI, int na, int nv);
+size_t hessian_diagonal_ws_bytes(int ld, int nI);
+size_t krylov_ws_bytes(int64_t n, int k);
 
 }  // namespace oo

@@ -107,9 +107,6 @@ struct TnArgs {
     uint32_t zero;
 };
 
-struct FalseTag { static constexpr bool value = false; };
-struct TrueTag { static constexpr bool value = true; };
-
 // shared -> global bulk asynchronous copy (TMA store path; tracked by the issuing thread's bulk group)
 __device__ __forceinline__ void bulk_store_1d(void *gdst, uint32_t smem_src, uint32_t bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_src), "r"(bytes)

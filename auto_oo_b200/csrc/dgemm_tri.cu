@@ -21,9 +21,6 @@
 
 namespace oo {
 
-int encode_tmap_4d_f64(CUtensorMap *map, const void *base, const uint64_t dims[4], const uint64_t strides_elems[3],
-                       const uint32_t box[4]);
-
 namespace {
 
 // MTC_: 8-row MMA tiles per group that hold class indices (ceil(nclass / 8) <= GP / 8); tiles past it are padding
@@ -61,9 +58,6 @@ struct TriArgs {
     int last_subs;          // substeps of the last k-block with rows below K
     uint32_t zero;
 };
-
-struct FalseTag { static constexpr bool value = false; };
-struct TrueTag { static constexpr bool value = true; };
 
 __device__ __forceinline__ void tma_load_4d(void *smem_dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1,
                                             int c2, int c3) {

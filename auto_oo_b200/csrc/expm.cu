@@ -22,11 +22,6 @@
 
 namespace oo {
 
-int dgemm_small(int transA, int transB, int M, int N, int K, double alpha, const double *A, int lda,
-                int64_t strideA, const double *B, int ldb, int64_t strideB, double beta,
-                const double *E, int lde, int64_t strideE, double gamma, double *D, int ldd,
-                int64_t strideD, int batch, cudaStream_t stream, int eye_n);
-
 namespace {
 
 // A[b] = scale * K(kappa[b]):  K[l,r] = +kappa_j, K[r,l] = -kappa_j

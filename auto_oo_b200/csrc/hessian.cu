@@ -18,84 +18,18 @@
 // is combined four ways directly into the (nk x nk) output.
 // B is the class buffer of classes.cu (or is gathered into that layout from the complete g').  At is not dense:
 // it splits into the C block (one TN-DGEMM), one G block per occupied orbital (bulk-async streamed DMMA kernel)
-// and an ELL remainder -- see "block structure of At" below; OO_FLAG_HESSIAN_DENSE keeps the single dense GEMM
-// over all of At for A/B tests.  The assembly is row-tiled and, for the rows outside I, streamed with bulk copies.
+// and an ELL remainder -- see "block structure of At" in hessian_terms.cuh; OO_FLAG_HESSIAN_DENSE keeps the single
+// dense GEMM over all of At for A/B tests.  The assembly is row-tiled and, for the rows outside I, streamed with bulk
+// copies.
 #include <stdlib.h>
 
-#include "common.cuh"
+#include "hessian_terms.cuh"
 
 namespace oo {
 
-
-int dgemm_tn(const double *At, const double *B, double *C, int64_t M, int64_t N, int64_t K,
-             int64_t lda, int64_t ldb, int64_t ldc, int batch, int64_t strideA, int64_t strideB,
-             int64_t strideC, cudaStream_t stream);
-
 namespace {
 
-struct RdmView {
-    const double *d1, *d2;
-    int no, na;
-};
-
-// full-space 1-RDM on I x I  (oo_energy.py:359-361)
-__device__ __forceinline__ double gf1(const RdmView &r, int p, int q) {
-    if (p >= r.no + r.na || q >= r.no + r.na) return 0.0;
-    if (p < r.no || q < r.no) return (p == q) ? 2.0 : 0.0;
-    return r.d1[(p - r.no) * r.na + (q - r.no)];
-}
-
-// full-space 2-RDM on I^4  (oo_energy.py:363-378)
-__device__ __forceinline__ double gf2(const RdmView &r, int p, int q, int s, int t) {
-    const int no = r.no, na = r.na;
-    const int nI = no + na;
-    if (p >= nI || q >= nI || s >= nI || t >= nI) return 0.0;
-    const bool op = p < no, oq = q < no, os = s < no, ot = t < no;
-    const int code = (op ? 8 : 0) | (oq ? 4 : 0) | (os ? 2 : 0) | (ot ? 1 : 0);
-    switch (code) {
-        case 15:  // occ occ occ occ : 4 d_pq d_st - 2 d_pt d_qs
-            return (p == q && s == t ? 4.0 : 0.0) - (p == t && q == s ? 2.0 : 0.0);
-        case 12:  // occ occ act act : 2 gamma_st d_pq
-            return p == q ? 2.0 * r.d1[(s - no) * na + (t - no)] : 0.0;
-        case 3:   // act act occ occ : 2 gamma_pq d_st
-            return s == t ? 2.0 * r.d1[(p - no) * na + (q - no)] : 0.0;
-        case 9:   // occ act act occ : -gamma_qs d_pt
-            return p == t ? -r.d1[(q - no) * na + (s - no)] : 0.0;
-        case 6:   // act occ occ act : -gamma_tp d_qs
-            return q == s ? -r.d1[(t - no) * na + (p - no)] : 0.0;
-        case 0:   // act act act act
-            return r.d2[(((int64_t)(p - no) * na + (q - no)) * na + (s - no)) * na + (t - no)];
-        default:
-            return 0.0;
-    }
-}
-
-// At rows: [0,nI^2) exchange-type, [nI^2, 2nI^2) Coulomb-type, 2nI^2: one-body.  lda >= nI^2 (even).
-// nI here is the ROW STRIDE of the I-space (nI for the full-tensor path, nIp for the class path;
-// gf1/gf2 return 0 for indices beyond occ+act).  swap_exch: exchange rows are ordered (n,m)
-// instead of (m,n) -- the order in which classes.cu stores K[n,m,a,b].
-// At[k, (p r)]: k < nI^2 exchange row (m,n) -- or (n,m) when swap_exch --, k < 2 nI^2 Coulomb row (m,n),
-// k = 2 nI^2 the one-body row.  `mn` receives the (m, n) the row stands for (-1 for the one-body row).
-__device__ __forceinline__ double at_value(const RdmView &rdm, int nI, int swap_exch, int64_t k, int p, int r,
-                                           int &m, int &n) {
-    const int nI2 = nI * nI;
-    if (k < nI2) {
-        const int k1 = (int)(k / nI), k2 = (int)(k % nI);
-        m = swap_exch ? k2 : k1;
-        n = swap_exch ? k1 : k2;
-        return 2.0 * (gf2(rdm, p, m, r, n) + gf2(rdm, p, m, n, r));
-    }
-    if (k < 2 * nI2) {
-        const int kk = (int)(k - nI2);
-        m = kk / nI;
-        n = kk % nI;
-        return 2.0 * gf2(rdm, p, r, m, n);
-    }
-    m = n = -1;
-    return 2.0 * gf1(rdm, p, r);
-}
-
-__global__ void hess_build_at_kernel(RdmView rdm, int nI, int swap_exch, int64_t lda, double *__restrict__ At) {
+__global__ void hess_build_at_kernel(RdmView rdm, int nI, int64_t lda, double *__restrict__ At) {
     const int nI2 = nI * nI;
     const int64_t total = (int64_t)(2 * nI2 + 1) * lda;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -104,86 +38,14 @@ __global__ void hess_build_at_kernel(RdmView rdm, int nI, int swap_exch, int64_t
         const int col = (int)(i % lda);
         double v = 0.0;
         int m, n;
-        if (col < nI2) v = at_value(rdm, nI, swap_exch, k, col / nI, col % nI, m, n);
+        if (col < nI2) v = at_value(rdm, nI, k, col / nI, col % nI, m, n);
         At[i] = v;
     }
 }
 
-// ---- block structure of At (class path) -------------------------------------------------------
-// The full-space 2-RDM is a dense na^4 block plus Kronecker-delta core blocks (full_rdms,
-// oo_energy.py:356-379), so At = [dense blocks] + [O(1) entries per column]:
-//   C block  columns: the na^2 act-act pairs (t u) and the no occupied diagonal pairs (i i);
-//            rows:    exchange / Coulomb rows of the act-act pairs and of the occupied diagonal pairs, one-body row
-//            (Gamma_tuvw, and the delta_ij gamma / delta_ij delta_kl terms summed over a whole class)
-//            -> ONE TN-DGEMM  Tc = Atc^T Bc  on the tensor pipe                    (~4 (na^2+no)^2 N^2 flop)
-//   G block of every occupied i   columns: (i t) and (t i), t active;
-//            rows: exchange / Coulomb rows at the positions (i u) and (u i), u active (the gamma_tu delta_ij terms)
-//            -> hess_group_kernel: the 4 na rows are read once per column chunk, 2 na x 4 na coefficients in smem
-//   rest     (occ-occ pairs i != j: three entries per column) -> ELL SpMM (hess_spmm_kernel), which also adds
-//            whatever a column of the two blocks has outside its block (nothing for the reference's RDM layout).
-// Every coefficient comes from the same at_value() as the all-dense route; a row k is identified by its
-// position pair (a, b) = ((k mod nIs^2) / nIs, (k mod nIs^2) mod nIs), which makes the row sets independent of
-// the storage order of the exchange rows.
-struct Blocks {
-    int no, na, nIs;
-    __device__ __host__ int ncol_c() const { return na * na + no; }
-    __device__ __host__ int nrow_c() const { return 2 * (na * na + no) + 1; }
-    __device__ __host__ int ncol_g() const { return 2 * na; }
-    __device__ __host__ int nrow_g() const { return 4 * na; }
-    // column cc of the C block -> (p, r)
-    __device__ void col_c(int cc, int &p, int &r) const {
-        if (cc < na * na) { p = no + cc / na; r = no + cc % na; } else { p = r = cc - na * na; }
-    }
-    // row kc of the C block -> row of At / B
-    __device__ int64_t row_c(int kc) const {
-        const int nC = na * na + no;
-        const int64_t nI2 = (int64_t)nIs * nIs;
-        if (kc >= 2 * nC) return 2 * nI2;
-        const int j = kc % nC;
-        const int a = j < na * na ? no + j / na : j - na * na, b = j < na * na ? no + j % na : j - na * na;
-        return (kc >= nC ? nI2 : 0) + (int64_t)a * nIs + b;
-    }
-    // column e of the G block of occupied i -> (p, r);  row kg -> row of At / B
-    __device__ void col_g(int i, int e, int &p, int &r) const {
-        if (e < na) { p = i; r = no + e; } else { p = no + e - na; r = i; }
-    }
-    __device__ int64_t row_g(int i, int kg) const {
-        const int u = no + kg % na, part = kg / na;              // 0: exch (i u), 1: exch (u i), 2: coul (i u), 3: coul (u i)
-        const int a = (part & 1) ? u : i, b = (part & 1) ? i : u;
-        return (part >= 2 ? (int64_t)nIs * nIs : 0) + (int64_t)a * nIs + b;
-    }
-    // home of column (p, r): 1 = C block, 2 = G block, 0 = none (ELL only)
-    __device__ int home(int p, int r) const {
-        const int nI = no + na;
-        if (p >= nI || r >= nI) return 0;
-        const bool po = p < no, ro = r < no;
-        if (!po && !ro) return 1;
-        if (po && ro) return p == r ? 1 : 0;
-        return 2;
-    }
-    // is entry (row k, column (p r)) part of the column's dense block?
-    __device__ bool covered(int p, int r, int64_t k) const {
-        const int h = home(p, r);
-        if (h == 0) return false;
-        const int64_t nI2 = (int64_t)nIs * nIs;
-        const int nI = no + na;
-        if (k == 2 * nI2) return h == 1;
-        const int kk = (int)(k % nI2), a = kk / nIs, b = kk % nIs;
-        if (a >= nI || b >= nI) return false;
-        if (h == 1) return (a >= no && b >= no) || (a == b && a < no);
-        const int i = p < no ? p : r;
-        return (a == i && b >= no) || (b == i && a >= no);
-    }
-    // offset (in rows of ld^2 doubles) of column (p, r) inside its block's result buffer
-    __device__ int64_t slot_c(int p, int r) const { return p < no ? na * na + p : (p - no) * na + (r - no); }
-    __device__ int64_t slot_g(int p, int r) const {
-        return p < no ? (int64_t)p * 2 * na + (r - no) : (int64_t)r * 2 * na + na + (p - no);
-    }
-};
-
 // one warp per column (p r) of At: ELL list (k, val) of its non-zeros outside the dense block
 __global__ void __launch_bounds__(256)
-hess_sparse_build_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int swap_exch, int width,
+hess_sparse_build_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int width,
                          int *__restrict__ cnt, int *__restrict__ idx, double *__restrict__ val,
                          int *__restrict__ overflow) {
     const int lane = threadIdx.x & 31;
@@ -204,7 +66,7 @@ hess_sparse_build_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int sw
             double v = 0.0;
             if (k < krows) {
                 int m, n;                                  // (block entries are not even evaluated: no Gamma loads here)
-                if (!Blocks{rdm.no, rdm.na, nIs}.covered(p, r, k)) v = at_value(rdm, nIs, swap_exch, k, p, r, m, n);
+                if (!Blocks{rdm.no, rdm.na, nIs}.covered(p, r, k)) v = at_value(rdm, nIs, k, p, r, m, n);
             }
             const unsigned mask = __ballot_sync(0xffffffffu, v != 0.0);
             if (v != 0.0) {
@@ -223,7 +85,7 @@ hess_sparse_build_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int sw
 }
 
 // C block operands: Atc[kc, cc] and Bc[kc, :] = the matching row of the class buffer
-__global__ void hess_dense_at_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int swap_exch, int64_t lda,
+__global__ void hess_dense_at_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int nIs, int64_t lda,
                                      double *__restrict__ Atc) {
     const RdmView rdm{rdm0.d1 + blockIdx.y * sd1, rdm0.d2 + blockIdx.y * sd2, rdm0.no, rdm0.na};
     const Blocks bl{rdm.no, rdm.na, nIs};
@@ -236,7 +98,7 @@ __global__ void hess_dense_at_kernel(RdmView rdm0, int64_t sd1, int64_t sd2, int
         if (cc < bl.ncol_c()) {
             int p, r, m, n;
             bl.col_c(cc, p, r);
-            v = at_value(rdm, nIs, swap_exch, bl.row_c(kc), p, r, m, n);
+            v = at_value(rdm, nIs, bl.row_c(kc), p, r, m, n);
         }
         Atc[i] = v;
     }
@@ -262,7 +124,7 @@ __global__ void hess_dense_b_kernel(const double *__restrict__ cls, int64_t cls_
 template <int CH>
 __global__ void __launch_bounds__(128)
 hess_group_kernel(const double *__restrict__ B, int64_t b_stride, RdmView rdm0, int64_t sd1, int64_t sd2,
-                  int rdm_batched, int nIs, int swap_exch, int64_t mat, double *__restrict__ Tg) {
+                  int rdm_batched, int nIs, int64_t mat, double *__restrict__ Tg) {
     extern __shared__ __align__(16) double coef[];                 // [4 na][2 na] then int64 row offsets [4 na]
     const int bz = blockIdx.z;
     const RdmView rdm{rdm0.d1 + (rdm_batched ? bz * sd1 : 0), rdm0.d2 + (rdm_batched ? bz * sd2 : 0), rdm0.no,
@@ -273,7 +135,7 @@ hess_group_kernel(const double *__restrict__ B, int64_t b_stride, RdmView rdm0, 
     for (int x = threadIdx.x; x < nr * nc; x += blockDim.x) {
         int p, r, m, n;
         bl.col_g(i, x % nc, p, r);
-        coef[x] = at_value(rdm, nIs, swap_exch, bl.row_g(i, x / nc), p, r, m, n);
+        coef[x] = at_value(rdm, nIs, bl.row_g(i, x / nc), p, r, m, n);
     }
     for (int x = threadIdx.x; x < nr; x += blockDim.x) rowoff[x] = bl.row_g(i, x) * mat;
     __syncthreads();
@@ -339,7 +201,7 @@ constexpr int kGrpMT = kGrpTile / kGrpWarps / 8;
 template <int NT>                                   // result rows padded to 8 NT >= 2 na
 __global__ void __launch_bounds__(32 * kGrpWarps, 1)
 hess_group_stream_kernel(const double *__restrict__ B, int64_t b_stride, RdmView rdm0, int64_t sd1, int64_t sd2,
-                         int rdm_batched, int nIs, int swap_exch, int64_t mat, double *__restrict__ Tg,
+                         int rdm_batched, int nIs, int64_t mat, double *__restrict__ Tg,
                          int tiles_per_i, int items_per_cta) {
     extern __shared__ __align__(128) unsigned char gs_smem[];
     const int bz = blockIdx.y;
@@ -388,7 +250,7 @@ hess_group_stream_kernel(const double *__restrict__ B, int64_t b_stride, RdmView
                 if (e < nc) {
                     int p, r, m, n;
                     bl.col_g(i, e, p, r);
-                    v = at_value(rdm, nIs, swap_exch, bl.row_g(i, kg), p, r, m, n);
+                    v = at_value(rdm, nIs, bl.row_g(i, kg), p, r, m, n);
                 }
                 coef[kg * CS + e] = v;
             }
@@ -580,32 +442,6 @@ hess_spmm_pair_kernel(const double *__restrict__ B, int64_t b_stride, const int 
             *reinterpret_cast<double2 *>(T + (int64_t)col0 * mat + c) = a0[u];
             *reinterpret_cast<double2 *>(T + (int64_t)col1 * mat + c) = a1[u];
         }
-    }
-}
-
-// B rows as above; columns (q s) over ld x ld (padding columns come out as the zero padding of g, h).
-__global__ void hess_gather_b_kernel(const double *__restrict__ h, const double *__restrict__ g, int nI,
-                                     int ld, double *__restrict__ B) {
-    const int nI2 = nI * nI;
-    const int64_t mat = (int64_t)ld * ld;
-    const int64_t total = (int64_t)(2 * nI2 + (h ? 1 : 0)) * mat;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
-        const int64_t k = i / mat;
-        const int64_t c = i % mat;
-        const int q = (int)(c / ld), s = (int)(c % ld);
-        double v;
-        if (k < nI2) {
-            const int m = (int)(k / nI), n = (int)(k % nI);
-            v = g[(((int64_t)q * ld + m) * ld + n) * ld + s];
-        } else if (k < 2 * nI2) {
-            const int kk = (int)(k - nI2);
-            const int m = kk / nI, n = kk % nI;
-            v = g[(((int64_t)q * ld + s) * ld + m) * ld + n];
-        } else {
-            v = h[c];
-        }
-        B[i] = v;
     }
 }
 
@@ -937,6 +773,24 @@ __global__ void y_build_at_kernel(const double *__restrict__ G, int N, int64_t l
     }
 }
 
+// B rows of the same product: [0,N^2) exchange rows (m n) g[q,m,n,s], [N^2, 2N^2) Coulomb rows (m n) g[q,s,m,n];
+// columns (q s) over ld x ld (padding columns come out as the zero padding of g)
+__global__ void y_gather_b_kernel(const double *__restrict__ g, int nI, int ld, double *__restrict__ B) {
+    const int nI2 = nI * nI;
+    const int64_t mat = (int64_t)ld * ld;
+    const int64_t total = (int64_t)(2 * nI2) * mat;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        const int64_t k = i / mat;
+        const int64_t c = i % mat;
+        const int q = (int)(c / ld), s = (int)(c % ld);
+        const bool exch = k < nI2;
+        const int kk = (int)(exch ? k : k - nI2);
+        const int m = kk / nI, n = kk % nI;
+        B[i] = exch ? g[(((int64_t)q * ld + m) * ld + n) * ld + s] : g[(((int64_t)q * ld + s) * ld + m) * ld + n];
+    }
+}
+
 // Y[p,q,r,s] (dense N^4) = T[(p r),(q s)] (row pitch ld*ld)
 __global__ void y_permute_kernel(const double *__restrict__ T, int N, int ld, double *__restrict__ Y) {
     const int64_t n2 = (int64_t)N * N, n4 = n2 * n2;
@@ -1007,15 +861,6 @@ HessLayout hess_layout(int ld, int nI) {
     return L;
 }
 
-}  // namespace
-
-int class_hessian(const double *cls, const double *F, const double *d1, int64_t sd1, const double *d2,
-                  int64_t sd2, int no, int na, int N, int ld, int nIp, int batch, const int32_t *pl,
-                  const int32_t *pr, int nk, double *H, void *ws, size_t ws_bytes, unsigned flags,
-                  cudaStream_t stream);
-size_t class_hessian_ws_bytes(int ld, int nIp, int no, int na, int batch);
-
-namespace {
 // class-layout B operand from the complete tensor: rows [K(n,m) | J(m,n) | h], m, n < nIp (zero rows beyond nI)
 //   K[n,m,a,b] = g'[a,m,n,b],  J[m,n,a,b] = g'[a,b,m,n]   (the layout classes.cu produces)
 __global__ void hess_gather_class_kernel(const double *__restrict__ h, const double *__restrict__ g, int nI, int nIp,
@@ -1040,10 +885,22 @@ __global__ void hess_gather_class_kernel(const double *__restrict__ h, const dou
     }
 }
 
+}  // namespace
+
 size_t full_hessian_b_bytes(int ld, int nIp) {
     return align_up((size_t)(2 * (size_t)nIp * nIp + 1) * ld * ld * sizeof(double), 1024);
 }
-}  // namespace
+
+// the class layout gathered out of the complete g' into B (full_hessian_b_bytes): the (h', g') forms of the Hessian,
+// its product and its diagonal run the class-buffer kernels on it
+int gather_class_layout(const double *h, const double *g, int nI, int ld, double *B, cudaStream_t stream) {
+    const int nIp = nI + (nI & 1);
+    int64_t blocks = ceil_div((2 * (int64_t)nIp * nIp + 1) * ld * ld, 256);
+    if (blocks > 16 * sm_count()) blocks = 16 * sm_count();
+    hess_gather_class_kernel<<<(unsigned)blocks, 256, 0, stream>>>(h, g, nI, nIp, ld, B);
+    OO_LAUNCH_CHECK();
+    return OO_OK;
+}
 
 // workspace of oo_hessian_f64: the gathered class-layout operand + the class Hessian's own workspace (largest over
 // the occ / act splits of nI, which this query does not know)
@@ -1072,11 +929,8 @@ int hessian(const double *h, const double *g, const double *F, const double *d1,
     if (nk > 65535) return OO_ERR_UNSUPPORTED;
     uint8_t *w = reinterpret_cast<uint8_t *>(ws);
     double *B = reinterpret_cast<double *>(w);
-    const int64_t mat = (int64_t)ld * ld;
-    int64_t blocks = ceil_div((2 * (int64_t)nIp * nIp + 1) * mat, 256);
-    if (blocks > 16 * sm_count()) blocks = 16 * sm_count();
-    hess_gather_class_kernel<<<(unsigned)blocks, 256, 0, stream>>>(h, g, nI, nIp, ld, B);
-    OO_LAUNCH_CHECK();
+    int rc = gather_class_layout(h, g, nI, ld, B, stream);
+    if (rc) return rc;
     return class_hessian(B, F, d1, 0, d2, 0, no, na, N, ld, nIp, 1, pl, pr, nk, H, w + b_bytes, c_bytes, flags,
                          stream);
 }
@@ -1091,7 +945,7 @@ struct ClassHessLayout {
 static ClassHessLayout class_hess_layout(int ld, int nIp, int no, int na, int batch) {
     ClassHessLayout L;
     const int64_t nI2 = (int64_t)nIp * nIp, mat = (int64_t)ld * ld, na2 = (int64_t)na * na;
-    L.width = 2 * na * na + 2 * (no + na) + 8;
+    L.width = ell_width(no, na);
     L.ncol_c = na2 + no;
     L.lda_c = (L.ncol_c + 1) & ~1ll;
     L.krows_c = 2 * L.ncol_c + 1;
@@ -1128,7 +982,7 @@ static int class_hessian_dense(const double *cls, const double *F, const RdmView
     const int64_t nI2 = (int64_t)nIp * nIp, mat = (int64_t)ld * ld;
     int64_t blocks = ceil_div(L.krows * L.lda, 256);
     if (blocks > 8 * sm_count()) blocks = 8 * sm_count();
-    hess_build_at_kernel<<<(unsigned)blocks, 256, 0, stream>>>(rdm, nIp, 1, L.lda, At);
+    hess_build_at_kernel<<<(unsigned)blocks, 256, 0, stream>>>(rdm, nIp, L.lda, At);
     OO_LAUNCH_CHECK();
     int rc = dgemm_tn(At, cls, T, nI2, mat, L.krows, L.lda, mat, mat, 1, 0, 0, 0, stream);
     if (rc) return rc;
@@ -1182,14 +1036,14 @@ int class_hessian(const double *cls, const double *F, const double *d1, int64_t 
     // ELL lists of what lies outside the dense blocks (one table per set of RDMs)
     if (!reuse) {
         hess_sparse_build_kernel<<<dim3((unsigned)ceil_div(nI2, 8), (unsigned)nsets), 256, 0, stream>>>(
-            rdm, sd1, sd2, nIp, 1, L.width, cnt, idx, val, flag);
+            rdm, sd1, sd2, nIp, L.width, cnt, idx, val, flag);
         OO_LAUNCH_CHECK();
     }
     // C block: Tc[b] = Atc^T Bc[b]
     {
         int64_t blocks = ceil_div(L.krows_c * L.lda_c, 256);
         if (!reuse) {
-            hess_dense_at_kernel<<<dim3((unsigned)blocks, (unsigned)nsets), 256, 0, stream>>>(rdm, sd1, sd2, nIp, 1,
+            hess_dense_at_kernel<<<dim3((unsigned)blocks, (unsigned)nsets), 256, 0, stream>>>(rdm, sd1, sd2, nIp,
                                                                                              L.lda_c, Atc);
             OO_LAUNCH_CHECK();
         }
@@ -1222,7 +1076,7 @@ int class_hessian(const double *cls, const double *F, const double *d1, int64_t 
             OO_CUDA_CHECK(cudaFuncSetAttribute(hess_group_stream_kernel<CH>,                                       \
                                                cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));          \
         hess_group_stream_kernel<CH><<<sgrid, 32 * kGrpWarps, smem_stream, stream>>>(cls, cls_stride, rdm, sd1, sd2,          \
-                                                                         rdm_batched, nIp, 1, mat, Tg,             \
+                                                                         rdm_batched, nIp, mat, Tg,                \
                                                                          tiles_per_i, items);                     \
     } while (0)
             if (2 * na <= 8) OO_GROUP_STREAM(1);
@@ -1232,7 +1086,7 @@ int class_hessian(const double *cls, const double *F, const double *d1, int64_t 
         } else {
         dim3 grid((unsigned)no, (unsigned)ceil_div(mat / 2, 128), (unsigned)batch);
 #define OO_GROUP(CH) hess_group_kernel<CH><<<grid, 128, smem, stream>>>(cls, cls_stride, rdm, sd1, sd2, rdm_batched, \
-                                                                       nIp, 1, mat, Tg)
+                                                                       nIp, mat, Tg)
         // (measured at N = 256, na = 12: 8 / 12 / 24 columns per pass all take 0.48-0.51 ms -- DRAM latency bound)
         if (2 * na <= 8) OO_GROUP(8);
         else if (2 * na <= 16) OO_GROUP(16);
@@ -1344,7 +1198,7 @@ int y_matrix(const double *g, const double *two_full, int N, int ld, double *Y, 
     OO_LAUNCH_CHECK();
     blocks = ceil_div(2 * N2 * mat, 256);
     if (blocks > 16 * sm_count()) blocks = 16 * sm_count();
-    hess_gather_b_kernel<<<(unsigned)blocks, 256, 0, stream>>>(nullptr, g, N, ld, B);
+    y_gather_b_kernel<<<(unsigned)blocks, 256, 0, stream>>>(g, N, ld, B);
     OO_LAUNCH_CHECK();
     int rc = dgemm_tn(At, B, T, N2, mat, 2 * N2, L.lda, mat, mat, 1, 0, 0, 0, stream);
     if (rc) return rc;
@@ -1355,420 +1209,7 @@ int y_matrix(const double *g, const double *two_full, int N, int ld, double *Y, 
     return OO_OK;
 }
 
-// ---- matrix-free Hessian: H v and diag(H) straight from the class buffer ----------------------------------------------
-// For a block of vectors v (nk) let V be the skew matrix of each, V[l_j, r_j] = v_j = -V[r_j, l_j].  Then
-//   W[p,q]  = -((F + F^T) V)[p,q] + [p in I] sum_{r in I, s} T[(p r),(q s)] V[r,s],      (H v)_j = W[l_j,r_j] - W[r_j,l_j]
-// and with A_k[p,r] = At[k,(p r)] (at_value) the T part is
-//   sum_k sum_s B[k][q,s] M_k[p,s],   M_k[p,s] = sum_r A_k[p,r] V[r,s]:
-// every class plane B[k] is read once per block of vectors and multiplied (DMMA) by the few rows M_k has; neither T
-// nor the nk x nk matrix is formed.  The diagonal needs four T elements per parameter, each a dot product of a column
-// of At with one element of every plane.
-namespace {
-
-constexpr int kHvpQT = 32;                          // q rows per CTA tile (4 DMMA row tiles)
-constexpr int kHvpSC = 32;                          // s columns per CTA tile (8 DMMA k-steps)
-constexpr int kHvpSR = kHvpSC + 4;                  // shared-memory row stride (= 4 mod 32: conflict-free fragments)
-constexpr int kHvpStages = 4;                       // class-plane tiles in flight per CTA
-constexpr int kHvpMaxVec = 8;                       // vectors per pass at most
-constexpr int kHvpCtas = 592;                       // target grid (a fixed number: the summation order, and with it every
-                                                    // bit of the result, does not depend on the device)
-constexpr size_t kHvpSmemMax = 200 * 1024;
-
-// Non-zeros of one class row of At.  From the Kronecker structure of the full-space RDMs (gf1 / gf2) a row has at
-// most na^2 + no + 4 of them (the act-act block, the occupied diagonal and a few occ-occ terms), below the width
-// of the ELL table the T-matrix build uses; that width is kept here.
-int hvp_width(int no, int na) { return 2 * na * na + 2 * (no + na) + 8; }
-
-struct HvpLayout {
-    int nvc, width, kc, rows_per, nsc, nqt;
-    size_t smem, off_np, off_plist, off_pstart, off_er, off_ev, off_part, off_v, off_w, total;
-};
-
-size_t hvp_smem_bytes(int nI, int nvc) {
-    const size_t ncol = (size_t)nI * nvc;
-    return ((size_t)kHvpStages * kHvpQT * kHvpSR + ncol * kHvpSR + (ncol + 7) / 8 * 8 * kHvpSR +
-            (size_t)nI * kHvpQT * nvc) * sizeof(double);
-}
-
-HvpLayout hvp_layout(int ld, int nIp, int no, int na, int nv) {
-    HvpLayout L;
-    const int nI = no + na;
-    const int64_t krows = 2 * (int64_t)nIp * nIp + 1, mat = (int64_t)ld * ld;
-    L.nvc = 0;
-    for (int c = 1; c <= kHvpMaxVec && c <= nv; ++c)
-        if (hvp_smem_bytes(nI, c) <= kHvpSmemMax) L.nvc = c;
-    L.smem = hvp_smem_bytes(nI, L.nvc > 0 ? L.nvc : 1);
-    L.width = hvp_width(no, na);
-    L.nqt = (int)ceil_div(ld, kHvpQT);
-    L.nsc = (int)ceil_div(ld, kHvpSC);
-    const int64_t tiles = (int64_t)L.nqt * L.nsc;
-    int64_t kc = ceil_div(kHvpCtas, tiles);
-    if (kc > krows) kc = krows;
-    L.rows_per = (int)ceil_div(krows, kc);
-    L.kc = (int)ceil_div(krows, L.rows_per);
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes, 1024); return o; };
-    L.off_np = take((size_t)krows * sizeof(int));
-    L.off_plist = take((size_t)krows * nI * sizeof(int));
-    L.off_pstart = take((size_t)krows * (nI + 1) * sizeof(int));
-    L.off_er = take((size_t)krows * L.width * sizeof(int));
-    L.off_ev = take((size_t)krows * L.width * sizeof(double));
-    const int nvc = L.nvc > 0 ? L.nvc : 1;
-    L.off_part = take((size_t)L.kc * L.nsc * nvc * nI * ld * sizeof(double));
-    L.off_v = take((size_t)nvc * mat * sizeof(double));
-    L.off_w = take((size_t)nvc * mat * sizeof(double));
-    L.total = off;
-    return L;
-}
-
-// One warp per class row k: its non-zero coefficients A_k[p,r] (p, r < nI) grouped by p -- the distinct p in
-// plist[k][0, np), the entries of the i-th in [pstart[k][i], pstart[k][i+1]) with column r and value.
-__global__ void __launch_bounds__(256)
-hvp_table_kernel(RdmView rdm, int nIp, int64_t krows, int width, int *__restrict__ npk, int *__restrict__ plist,
-                 int *__restrict__ pstart, int *__restrict__ er, double *__restrict__ ev) {
-    const int lane = threadIdx.x & 31;
-    const int64_t k = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (k >= krows) return;
-    const int nI = rdm.no + rdm.na;
-    int base = 0, np = 0;
-    for (int p = 0; p < nI; ++p) {
-        const int start = base;
-        for (int r0 = 0; r0 < nI; r0 += 32) {
-            const int r = r0 + lane;
-            double v = 0.0;
-            int m, n;
-            if (r < nI) v = at_value(rdm, nIp, 1, k, p, r, m, n);
-            const unsigned mask = __ballot_sync(0xffffffffu, v != 0.0);
-            const int pos = base + __popc(mask & ((1u << lane) - 1u));
-            if (v != 0.0 && pos < width) {
-                er[k * width + pos] = r;
-                ev[k * width + pos] = v;
-            }
-            base += __popc(mask);
-        }
-        if (base > start) {
-            if (lane == 0) {
-                plist[k * nI + np] = p;
-                pstart[k * (nI + 1) + np] = min(start, width);
-            }
-            ++np;
-        }
-    }
-    if (lane == 0) {
-        pstart[k * (nI + 1) + np] = min(base, width);
-        npk[k] = np;
-    }
-}
-
-// Vm[v][l_j][r_j] = V[j][v0 + v] = -Vm[v][r_j][l_j]  (Vm zeroed before)
-__global__ void hvp_scatter_kernel(const double *__restrict__ V, int nv, int v0, int nvc, const int32_t *__restrict__ pl,
-                                   const int32_t *__restrict__ pr, int nk, int ld, double *__restrict__ Vm) {
-    const int64_t total = (int64_t)nk * nvc, mat = (int64_t)ld * ld;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int j = (int)(i / nvc), v = (int)(i % nvc);
-        const double x = V[(int64_t)j * nv + v0 + v];
-        Vm[v * mat + (int64_t)pl[j] * ld + pr[j]] = x;
-        Vm[v * mat + (int64_t)pr[j] * ld + pl[j]] = -x;
-    }
-}
-
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc, uint32_t src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(src_bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// The streamed pass.  CTA (q tile, s tile; range of class rows): for every row k of its range, the 32 x 32 tile
-// B[k][q0.., s0..] arrives by cp.async in a four-stage ring, M_k[(p v), s] = sum_r A_k[p,r] V_v[r,s] is formed in
-// shared memory from the CTA's slice of V (rows r in I), U[q, (p v)] = sum_s B[k][q,s] M_k[(p v), s] runs on DMMA,
-// and U is added to the CTA's W[p][q][v] (each element by exactly one thread per row k: a fixed order).  The CTA
-// writes its W to its own slice of `part`; hvp_reduce_kernel sums the slices in a fixed order.
-__global__ void __launch_bounds__(256)
-hvp_plane_kernel(const double *__restrict__ cls, int ld, int nI, int64_t krows, int rows_per, int nsc, int nvc,
-                 const int *__restrict__ npk, const int *__restrict__ plist, const int *__restrict__ pstart,
-                 const int *__restrict__ er, const double *__restrict__ ev, int width, const double *__restrict__ Vm,
-                 double *__restrict__ part) {
-    extern __shared__ __align__(16) double hv_smem[];
-    const int ncol_max = nI * nvc;
-    double *stage = hv_smem;                                          // [stages][QT][SR]
-    double *Vs = stage + kHvpStages * kHvpQT * kHvpSR;                // [(r v)][SR]
-    double *Ms = Vs + (size_t)ncol_max * kHvpSR;                      // [(i v)][SR], rows padded to 8
-    double *Ws = Ms + (size_t)(ncol_max + 7) / 8 * 8 * kHvpSR;        // [p][QT][v]
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    const int qt = blockIdx.x / nsc, sc = blockIdx.x % nsc;
-    const int q0 = qt * kHvpQT, s0 = sc * kHvpSC;
-    const int64_t mat = (int64_t)ld * ld;
-    const int64_t k0 = (int64_t)blockIdx.y * rows_per, k1 = min(k0 + rows_per, krows);
-
-    for (int x = tid; x < ncol_max * kHvpSC; x += blockDim.x) {
-        const int row = x / kHvpSC, s = x % kHvpSC, r = row / nvc, v = row % nvc;
-        Vs[row * kHvpSR + s] = s0 + s < ld ? Vm[v * mat + (int64_t)r * ld + s0 + s] : 0.0;
-    }
-    for (int x = tid; x < nI * kHvpQT * nvc; x += blockDim.x) Ws[x] = 0.0;
-
-    auto issue = [&](int64_t k, int slot) {                           // 32 rows x 16 granules of 16 bytes
-        for (int x = tid; x < kHvpQT * kHvpSC / 2; x += blockDim.x) {
-            const int row = x / (kHvpSC / 2), c2 = 2 * (x % (kHvpSC / 2));
-            const int q = q0 + row, s = s0 + c2;
-            const bool ok = q < ld && s < ld;
-            cp_async16(stage + (slot * kHvpQT + row) * kHvpSR + c2, ok ? cls + k * mat + (int64_t)q * ld + s : cls,
-                       ok ? 16u : 0u);
-        }
-    };
-    for (int i = 0; i < kHvpStages - 1; ++i) {
-        if (k0 + i < k1) issue(k0 + i, i);
-        cp_async_commit();
-    }
-    for (int64_t k = k0; k < k1; ++k) {
-        const int it = (int)(k - k0), slot = it % kHvpStages;
-        if (k + kHvpStages - 1 < k1) issue(k + kHvpStages - 1, (it + kHvpStages - 1) % kHvpStages);
-        cp_async_commit();
-        cp_async_wait<kHvpStages - 1>();
-        const int np = npk[k], ncol = np * nvc, ncolp = (ncol + 7) & ~7;
-        __syncthreads();                                              // tile k visible; Vs / Ws initialised
-        for (int x = tid; x < ncolp * kHvpSC; x += blockDim.x) {
-            const int col = x / kHvpSC, s = x % kHvpSC;
-            double m = 0.0;
-            if (col < ncol) {
-                const int i = col / nvc, v = col % nvc;
-                const int e1 = pstart[k * (nI + 1) + i + 1];
-                for (int e = pstart[k * (nI + 1) + i]; e < e1; ++e)
-                    m = fma(ev[k * width + e], Vs[(er[k * width + e] * nvc + v) * kHvpSR + s], m);
-            }
-            Ms[col * kHvpSR + s] = m;
-        }
-        __syncthreads();
-        const double *st = stage + slot * kHvpQT * kHvpSR;
-        for (int w = warp; w < 4 * (ncolp / 8); w += 8) {
-            const int mt = w & 3, nt = w >> 2;
-            double c0 = 0.0, c1 = 0.0;
-#pragma unroll
-            for (int ks = 0; ks < kHvpSC / 4; ++ks)
-                dmma884(c0, c1, st[(8 * mt + g) * kHvpSR + 4 * ks + t], Ms[(8 * nt + g) * kHvpSR + 4 * ks + t]);
-#pragma unroll
-            for (int cc = 0; cc < 2; ++cc) {
-                const int col = 8 * nt + 2 * t + cc;
-                if (col < ncol) {
-                    const int p = plist[k * nI + col / nvc], v = col % nvc;
-                    Ws[(p * kHvpQT + 8 * mt + g) * nvc + v] += cc ? c1 : c0;
-                }
-            }
-        }
-        __syncthreads();                                              // stage slot and Ms free for reuse
-    }
-    cp_async_wait<0>();
-    __syncthreads();
-    double *out = part + (int64_t)(blockIdx.y * nsc + sc) * nvc * nI * ld;
-    for (int x = tid; x < nI * kHvpQT * nvc; x += blockDim.x) {
-        const int v = x % nvc, ql = (x / nvc) % kHvpQT, p = x / (nvc * kHvpQT);
-        if (q0 + ql < ld) out[((int64_t)v * nI + p) * ld + q0 + ql] = Ws[x];
-    }
-}
-
-// Wy[v][p][q] = sum over the slices of `part` (fixed order) for p in I, 0 elsewhere
-__global__ void hvp_reduce_kernel(const double *__restrict__ part, int nslices, int nvc, int nI, int ld,
-                                  double *__restrict__ Wy) {
-    const int64_t mat = (int64_t)ld * ld, total = nvc * mat, slice = (int64_t)nvc * nI * ld;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int v = (int)(i / mat), p = (int)((i % mat) / ld), q = (int)(i % ld);
-        double w = 0.0;
-        if (p < nI) {
-            const double *src = part + ((int64_t)v * nI + p) * ld + q;
-            for (int j = 0; j < nslices; ++j) w += src[j * slice];
-        }
-        Wy[i] = w;
-    }
-}
-
-// HV[j][v0 + v] = W[v][l_j][r_j] - W[v][r_j][l_j]
-__global__ void hvp_gather_kernel(const double *__restrict__ W, int nvc, const int32_t *__restrict__ pl,
-                                  const int32_t *__restrict__ pr, int nk, int ld, int nv, int v0,
-                                  double *__restrict__ HV) {
-    const int64_t total = (int64_t)nk * nvc, mat = (int64_t)ld * ld;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int j = (int)(i / nvc), v = (int)(i % nvc);
-        const double *Wv = W + v * mat;
-        HV[(int64_t)j * nv + v0 + v] = Wv[(int64_t)pl[j] * ld + pr[j]] - Wv[(int64_t)pr[j] * ld + pl[j]];
-    }
-}
-
-// One warp per parameter j = (l, r):
-//   H_jj = X(l,r,l,r) - X(l,r,r,l) - X(r,l,l,r) + X(r,l,r,l),  X(a,b,c,d) = -(F_ac + F_ca) d_bd + [a,c in I] T[(a c),(b d)]
-// with the four T elements summed over the class rows in lane order and reduced by warp_sum (a fixed order).
-__global__ void __launch_bounds__(256)
-hess_diag_kernel(const double *__restrict__ cls, const double *__restrict__ F, RdmView rdm, int nIp, int ld,
-                 const int32_t *__restrict__ pl, const int32_t *__restrict__ pr, int nk, double *__restrict__ diag) {
-    const int lane = threadIdx.x & 31;
-    const int j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (j >= nk) return;
-    const int l = pl[j], r = pr[j], nI = rdm.no + rdm.na;
-    const bool li = l < nI, ri = r < nI;
-    const int64_t krows = 2 * (int64_t)nIp * nIp + 1, mat = (int64_t)ld * ld;
-    const int64_t o_llrr = (int64_t)r * ld + r, o_lrrl = (int64_t)r * ld + l, o_rllr = (int64_t)l * ld + r,
-                  o_rrll = (int64_t)l * ld + l;
-    double t = 0.0;                                   // T[(l l),(r r)] - T[(l r),(r l)] - T[(r l),(l r)] + T[(r r),(l l)]
-    if (li || ri) {
-        for (int64_t k = lane; k < krows; k += 32) {
-            const double *Bk = cls + k * mat;
-            int m, n;
-            if (li) {
-                const double a = at_value(rdm, nIp, 1, k, l, l, m, n);
-                if (a != 0.0) t = fma(a, Bk[o_llrr], t);
-            }
-            if (li && ri) {
-                const double a = at_value(rdm, nIp, 1, k, l, r, m, n);
-                if (a != 0.0) t = fma(-a, Bk[o_lrrl], t);
-                const double b = at_value(rdm, nIp, 1, k, r, l, m, n);
-                if (b != 0.0) t = fma(-b, Bk[o_rllr], t);
-            }
-            if (ri) {
-                const double a = at_value(rdm, nIp, 1, k, r, r, m, n);
-                if (a != 0.0) t = fma(a, Bk[o_rrll], t);
-            }
-        }
-    }
-    t = warp_sum(t);
-    if (lane == 0) {
-        const double Fll = F[(int64_t)l * ld + l], Frr = F[(int64_t)r * ld + r];
-        const double Fx = l == r ? F[(int64_t)l * ld + r] + F[(int64_t)r * ld + l] : 0.0;
-        diag[j] = -2.0 * Fll + 2.0 * Fx - 2.0 * Frr + t;
-    }
-}
-
-}  // namespace
-
-size_t class_hessian_vector_ws_bytes(int ld, int nIp, int no, int na, int nv) {
-    return hvp_layout(ld, nIp, no, na, nv).total;
-}
-
-size_t hessian_vector_ws_bytes(int ld, int nI, int na, int nv) {
-    const int nIp = nI + (nI & 1);
-    return full_hessian_b_bytes(ld, nIp) + class_hessian_vector_ws_bytes(ld, nIp, nI - na, na, nv);
-}
-
-size_t hessian_diagonal_ws_bytes(int ld, int nI) { return full_hessian_b_bytes(ld, nI + (nI & 1)); }
-
-int dgemm_small(int transA, int transB, int M, int N, int K, double alpha, const double *A, int lda,
-                int64_t strideA, const double *B, int ldb, int64_t strideB, double beta,
-                const double *E, int lde, int64_t strideE, double gamma, double *D, int ldd,
-                int64_t strideD, int batch, cudaStream_t stream, int eye_n);
-
-// HV = H V for one evaluation: V, HV are nk x nv row-major.
-int class_hessian_vector(const double *cls, const double *F, const double *d1, const double *d2, int no, int na,
-                         int N, int ld, int nIp, const int32_t *pl, const int32_t *pr, int nk, const double *V,
-                         int nv, double *HV, void *ws, size_t ws_bytes, cudaStream_t stream) {
-    OO_REQUIRE(cls && F && d1 && d2 && V && HV && ws && pl && pr);
-    OO_REQUIRE(no >= 0 && na > 0 && no + na <= N && ld >= N && (ld % 2) == 0 && nk > 0 && nv > 0);
-    OO_REQUIRE(nIp >= no + na && (nIp % 2) == 0 && nIp <= ld);
-    const HvpLayout L = hvp_layout(ld, nIp, no, na, nv);
-    if (L.nvc == 0) return OO_ERR_UNSUPPORTED;
-    if (ws_bytes < L.total) return OO_ERR_WORKSPACE;
-    if (L.kc > 65535) return OO_ERR_UNSUPPORTED;
-    const int nI = no + na;
-    const int64_t krows = 2 * (int64_t)nIp * nIp + 1, mat = (int64_t)ld * ld;
-    uint8_t *w = reinterpret_cast<uint8_t *>(ws);
-    int *npk = reinterpret_cast<int *>(w + L.off_np);
-    int *plist = reinterpret_cast<int *>(w + L.off_plist);
-    int *pstart = reinterpret_cast<int *>(w + L.off_pstart);
-    int *er = reinterpret_cast<int *>(w + L.off_er);
-    double *ev = reinterpret_cast<double *>(w + L.off_ev);
-    double *part = reinterpret_cast<double *>(w + L.off_part);
-    double *Vm = reinterpret_cast<double *>(w + L.off_v);
-    double *Wm = reinterpret_cast<double *>(w + L.off_w);
-    const RdmView rdm{d1, d2, no, na};
-    hvp_table_kernel<<<(unsigned)ceil_div(krows, 8), 256, 0, stream>>>(rdm, nIp, krows, L.width, npk, plist, pstart,
-                                                                      er, ev);
-    OO_LAUNCH_CHECK();
-    static unsigned long long cfgd = 0;
-    if (once_per_device(cfgd))
-        OO_CUDA_CHECK(cudaFuncSetAttribute(hvp_plane_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)kHvpSmemMax));
-    const int cap = 4 * sm_count();
-    for (int v0 = 0; v0 < nv; v0 += L.nvc) {
-        const int nvc = nv - v0 < L.nvc ? nv - v0 : L.nvc;
-        OO_CUDA_CHECK(cudaMemsetAsync(Vm, 0, (size_t)nvc * mat * sizeof(double), stream));
-        int64_t blocks = ceil_div((int64_t)nk * nvc, 256);
-        hvp_scatter_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(V, nv, v0, nvc, pl, pr, nk, ld,
-                                                                                        Vm);
-        OO_LAUNCH_CHECK();
-        hvp_plane_kernel<<<dim3((unsigned)(L.nqt * L.nsc), (unsigned)L.kc), 256, hvp_smem_bytes(nI, nvc), stream>>>(
-            cls, ld, nI, krows, L.rows_per, L.nsc, nvc, npk, plist, pstart, er, ev, L.width, Vm, part);
-        OO_LAUNCH_CHECK();
-        blocks = ceil_div(nvc * mat, 256);
-        hvp_reduce_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(part, L.kc * L.nsc, nvc, nI, ld,
-                                                                                       Wm);
-        OO_LAUNCH_CHECK();
-        // W -= F V  and  W -= F^T V   (the one-body part of X, on the small DMMA GEMM; E aliases D)
-        for (int tr = 0; tr < 2; ++tr) {
-            int rc = dgemm_small(tr, 0, ld, ld, ld, -1.0, F, ld, 0, Vm, ld, mat, 1.0, Wm, ld, mat, 0.0, Wm, ld, mat,
-                                 nvc, stream, 0);
-            if (rc) return rc;
-        }
-        blocks = ceil_div((int64_t)nk * nvc, 256);
-        hvp_gather_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(Wm, nvc, pl, pr, nk, ld, nv, v0,
-                                                                                       HV);
-        OO_LAUNCH_CHECK();
-    }
-    return OO_OK;
-}
-
-int class_hessian_diagonal(const double *cls, const double *F, const double *d1, const double *d2, int no, int na,
-                           int N, int ld, int nIp, const int32_t *pl, const int32_t *pr, int nk, double *diag,
-                           cudaStream_t stream) {
-    OO_REQUIRE(cls && F && d1 && d2 && diag && pl && pr);
-    OO_REQUIRE(no >= 0 && na > 0 && no + na <= N && ld >= N && (ld % 2) == 0 && nk > 0);
-    OO_REQUIRE(nIp >= no + na && (nIp % 2) == 0 && nIp <= ld);
-    hess_diag_kernel<<<(unsigned)ceil_div(nk, 8), 256, 0, stream>>>(cls, F, RdmView{d1, d2, no, na}, nIp, ld, pl, pr,
-                                                                    nk, diag);
-    OO_LAUNCH_CHECK();
-    return OO_OK;
-}
-
-// (h', g') forms: the class layout is gathered out of the complete g' into the workspace (as oo_hessian_f64 does)
-static int gather_class_layout(const double *h, const double *g, int nI, int ld, double *B, cudaStream_t stream) {
-    const int nIp = nI + (nI & 1);
-    int64_t blocks = ceil_div((2 * (int64_t)nIp * nIp + 1) * ld * ld, 256);
-    if (blocks > 16 * sm_count()) blocks = 16 * sm_count();
-    hess_gather_class_kernel<<<(unsigned)blocks, 256, 0, stream>>>(h, g, nI, nIp, ld, B);
-    OO_LAUNCH_CHECK();
-    return OO_OK;
-}
-
-int hessian_vector(const double *h, const double *g, const double *F, const double *d1, const double *d2, int no,
-                   int na, int N, int ld, const int32_t *pl, const int32_t *pr, int nk, const double *V, int nv,
-                   double *HV, void *ws, size_t ws_bytes, cudaStream_t stream) {
-    OO_REQUIRE(h && g && F && d1 && d2 && V && HV && ws && pl && pr);
-    OO_REQUIRE(no >= 0 && na > 0 && no + na <= N && ld >= N && (ld % 2) == 0 && nk > 0 && nv > 0);
-    const int nI = no + na, nIp = nI + (nI & 1);
-    const size_t b_bytes = full_hessian_b_bytes(ld, nIp);
-    if (ws_bytes < b_bytes) return OO_ERR_WORKSPACE;
-    uint8_t *w = reinterpret_cast<uint8_t *>(ws);
-    const HvpLayout L = hvp_layout(ld, nIp, no, na, nv);
-    if (L.nvc == 0) return OO_ERR_UNSUPPORTED;
-    if (ws_bytes < b_bytes + L.total) return OO_ERR_WORKSPACE;
-    int rc = gather_class_layout(h, g, nI, ld, reinterpret_cast<double *>(w), stream);
-    if (rc) return rc;
-    return class_hessian_vector(reinterpret_cast<double *>(w), F, d1, d2, no, na, N, ld, nIp, pl, pr, nk, V, nv, HV,
-                                w + b_bytes, ws_bytes - b_bytes, stream);
-}
-
-int hessian_diagonal(const double *h, const double *g, const double *F, const double *d1, const double *d2, int no,
-                     int na, int N, int ld, const int32_t *pl, const int32_t *pr, int nk, double *diag, void *ws,
-                     size_t ws_bytes, cudaStream_t stream) {
-    OO_REQUIRE(h && g && F && d1 && d2 && diag && ws && pl && pr);
-    OO_REQUIRE(no >= 0 && na > 0 && no + na <= N && ld >= N && (ld % 2) == 0 && nk > 0);
-    const int nI = no + na, nIp = nI + (nI & 1);
-    if (ws_bytes < full_hessian_b_bytes(ld, nIp)) return OO_ERR_WORKSPACE;
-    int rc = gather_class_layout(h, g, nI, ld, reinterpret_cast<double *>(ws), stream);
-    if (rc) return rc;
-    return class_hessian_diagonal(reinterpret_cast<double *>(ws), F, d1, d2, no, na, N, ld, nIp, pl, pr, nk, diag,
-                                  stream);
-}
-
 }  // namespace oo
-
 
 extern "C" int oo_hessian_f64(const double *h_mo, const double *g_mo, const double *F,
                               const double *gamma, const double *Gamma, int no, int na, int N, int ld,
@@ -1803,38 +1244,4 @@ extern "C" int oo_class_hessian_f64(const double *cls, const double *F, const do
                                     unsigned flags, void *stream) {
     return oo::class_hessian(cls, F, gamma, stride_rdm1, Gamma, stride_rdm2, no, na, N, ld, nIp, batch, pair_l,
                              pair_r, nk, H, ws, ws_bytes, flags, (cudaStream_t)stream);
-}
-
-extern "C" int oo_class_hessian_vector_f64(const double *cls, const double *F, const double *gamma,
-                                           const double *Gamma, int no, int na, int N, int ld, int nIp,
-                                           const int32_t *pair_l, const int32_t *pair_r, int nk, const double *V,
-                                           int nv, double *HV, void *ws, size_t ws_bytes, void *stream) {
-    return oo::class_hessian_vector(cls, F, gamma, Gamma, no, na, N, ld, nIp, pair_l, pair_r, nk, V, nv, HV, ws,
-                                    ws_bytes, (cudaStream_t)stream);
-}
-
-extern "C" int oo_class_hessian_diagonal_f64(const double *cls, const double *F, const double *gamma,
-                                             const double *Gamma, int no, int na, int N, int ld, int nIp,
-                                             const int32_t *pair_l, const int32_t *pair_r, int nk, double *diag,
-                                             void *ws, size_t ws_bytes, void *stream) {
-    (void)ws;
-    (void)ws_bytes;
-    return oo::class_hessian_diagonal(cls, F, gamma, Gamma, no, na, N, ld, nIp, pair_l, pair_r, nk, diag,
-                                      (cudaStream_t)stream);
-}
-
-extern "C" int oo_hessian_vector_f64(const double *h_mo, const double *g_mo, const double *F, const double *gamma,
-                                     const double *Gamma, int no, int na, int N, int ld, const int32_t *pair_l,
-                                     const int32_t *pair_r, int nk, const double *V, int nv, double *HV, void *ws,
-                                     size_t ws_bytes, void *stream) {
-    return oo::hessian_vector(h_mo, g_mo, F, gamma, Gamma, no, na, N, ld, pair_l, pair_r, nk, V, nv, HV, ws, ws_bytes,
-                              (cudaStream_t)stream);
-}
-
-extern "C" int oo_hessian_diagonal_f64(const double *h_mo, const double *g_mo, const double *F, const double *gamma,
-                                       const double *Gamma, int no, int na, int N, int ld, const int32_t *pair_l,
-                                       const int32_t *pair_r, int nk, double *diag, void *ws, size_t ws_bytes,
-                                       void *stream) {
-    return oo::hessian_diagonal(h_mo, g_mo, F, gamma, Gamma, no, na, N, ld, pair_l, pair_r, nk, diag, ws, ws_bytes,
-                                (cudaStream_t)stream);
 }

@@ -114,7 +114,7 @@ def test_odd_core_electrons_raises():
 @pytest.mark.parametrize("no,na", [(0, 3), (1, 2), (3, 4), (6, 4), (4, 6), (10, 3), (18, 6)])
 def test_hessian_sparse_row_bound(no, na):
     """The CUDA Hessian stores the non-dense part of At in ELL rows of width 2 na^2 + 2 (no+na) + 8
-    (csrc/hessian.cu, class_hess_layout).  Count the structural non-zeros of the reference's full-space
+    (csrc/hessian_terms.cuh, ell_width).  Count the structural non-zeros of the reference's full-space
     2-RDM (full_rdms, oo_energy.py:342-379) outside the act-act block and check the bound."""
     gen = torch.Generator().manual_seed(0)
     one = torch.rand(na, na, dtype=torch.float64, generator=gen) + 0.5          # no accidental zeros

@@ -27,7 +27,7 @@ from auto_oo_b200.synthetic import CONFIG_SHAPES, SyntheticMol, random_kappa, ra
 
 REPS = 25
 NVS = [1, 2, 4, 8, 16]
-PASS_VECTORS = 8            # vectors per streamed pass (csrc/hessian.cu kHvpMaxVec)
+PASS_VECTORS = 8            # vectors per streamed pass (csrc/hessian_operator.cu kHvpMaxVec)
 
 
 def timed(fn):
