@@ -155,6 +155,7 @@ size_t oo_workspace_bytes(int which, int N, int ld, int nI, int batch) {
             return (N > 0 && N <= nI) ? oo::hessian_vector_ws_bytes(ld, nI, N, batch) : 0;
         case OO_WS_HESSIAN_DIAGONAL: return oo::hessian_diagonal_ws_bytes(ld, nI);
         case OO_WS_KRYLOV: return oo::krylov_ws_bytes(N, nI);   /* N carries the vector length, nI the basis size */
+        case OO_WS_ROTATION_VJP: return oo::rotation_vjp_ws_bytes(ld, batch);
         default: return 0;
     }
 }

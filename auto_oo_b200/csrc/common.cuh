@@ -247,6 +247,7 @@ size_t full_hessian_b_bytes(int ld, int nIp);
 
 // workspace and buffer sizes (oo_workspace_bytes)
 size_t rotation_ws_bytes(int ld, int batch);
+size_t rotation_vjp_ws_bytes(int ld, int batch);
 size_t int1e_ws_bytes(int ld, int batch);
 size_t hessian_ws_bytes(int ld, int nI);
 size_t y_matrix_ws_bytes(int ld, int N);

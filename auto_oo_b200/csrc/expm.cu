@@ -354,28 +354,48 @@ struct ChainArgs {
     double *U;                    // (batch, ld, ld)
 };
 
-struct ChainProduct {             // D = X Y (+ B),  B = c0 I + c1 P1 + c2 P2 (+ c3 P3);  D2 = d0 I + d1 P1 + d2 D
+struct ChainProduct {             // D = X Y (+ X2 Y2) (+ B),  B = c0 I + c1 P1 + c2 P2 (+ c3 P3);  D2 = d0 I + d1 P1 + d2 D
     const double *X, *Y;
     double *D;
     const double *P1, *P2, *P3;
     double c0, c1, c2, c3;
     double *D2;
     double d0, d1, d2;
+    const double *X2, *Y2;        // second operand pair (the dual products of the Frechet chain), or nullptr
 };
 
-__device__ __forceinline__ void chain_tile(const ChainProduct &q, int b, int m0, int n0, int N, int ld, int K,
-                                           double *psm) {
+// acc = X[m0.., :] Y[:, n0..] of one 32 x 32 tile, staged whole (K <= PK_MAX); true for the warps that own the output
+__device__ __forceinline__ bool chain_tile_mma(const double *X, const double *Y, int64_t off, int m0, int n0, int ld,
+                                               int K, double *psm, double (&acc)[2][2][2]) {
     using namespace panel;
     const int K4 = (K + 3) & ~3;
-    const int64_t off = (int64_t)b * ld * ld;
     double *sA = psm, *sB = psm + TS * panel_ls(K);
-    stage_panel(sA, q.X + off, ld, true, m0, ld, K, K4);
-    stage_panel(sB, q.Y + off, ld, false, n0, ld, K, K4);
+    stage_panel(sA, X + off, ld, true, m0, ld, K, K4);
+    stage_panel(sB, Y + off, ld, false, n0, ld, K, K4);
     asm volatile("cp.async.commit_group;" ::: "memory");
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncthreads();
+    return tile_mma(sA, sB, true, false, K, K4, psm, acc);
+}
+
+__device__ __forceinline__ void chain_tile(const ChainProduct &q, int b, int m0, int n0, int N, int ld, int K,
+                                           double *psm) {
+    const int64_t off = (int64_t)b * ld * ld;
     double acc[2][2][2];
-    if (tile_mma(sA, sB, true, false, K, K4, psm, acc)) {
+    const bool own = chain_tile_mma(q.X, q.Y, off, m0, n0, ld, K, psm, acc);
+    if (q.X2) {
+        // second staging pass into the same panels (the reduction buffer of the first aliases them)
+        double acc2[2][2][2];
+        __syncthreads();
+        chain_tile_mma(q.X2, q.Y2, off, m0, n0, ld, K, psm, acc2);
+#pragma unroll
+        for (int i = 0; i < 2; ++i)
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+#pragma unroll
+                for (int c = 0; c < 2; ++c) acc[i][j][c] += acc2[i][j][c];
+    }
+    if (own) {
         const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
         const int g = lane >> 2, t = lane & 3;
         const int wm = ((warp & 3) >> 1) * 16, wn = (warp & 1) * 16;
@@ -414,33 +434,25 @@ __device__ __forceinline__ void chain_phase(const ChainProduct *q, int nprod, in
     }
 }
 
-__global__ void __launch_bounds__(panel::PTHREADS) expm_chain_kernel(const ChainArgs p) {
-    extern __shared__ __align__(16) double psm[];
-    cg::grid_group grid = cg::this_grid();
-    const int N = p.N, ld = p.ld, batch = p.batch;
-    const int64_t mat = (int64_t)ld * ld, sl = mat * batch;
-    double *A2 = p.ws + 0 * sl, *A3 = p.ws + 1 * sl, *A4 = p.ws + 2 * sl, *norms = p.ws + 3 * sl;
-    double *R0 = p.ws + 7 * sl, *T0 = p.ws + 8 * sl, *T1 = p.ws + 9 * sl, *A = p.ws + (int64_t)kExpmSlots * sl;
-    const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, gthreads = (int64_t)gridDim.x * blockDim.x;
-
-    // ---- phase 0: A = 0 (packed input) and, when s is ours to choose, ||sign * input_b||_1 per matrix
-    if (p.kappa)
-        for (int64_t i = gtid; i < sl; i += gthreads) A[i] = 0.0;
-    int squarings = p.squarings;
+// Phase 0 of the single-launch chains: the squaring count (s < 0: max over the batch of ceil(log2(||A_b||_1 / 0.95)),
+// from the packed kappa or the dense Ain), ending in a grid barrier either way.  Every CTA returns the same s.
+__device__ int chain_squarings(cg::grid_group &grid, const double *kappa, const int32_t *pl, const int32_t *pr, int nk,
+                               const double *Ain, int N, int ld, int batch, int squarings, double *norms, double *psm) {
+    const int64_t mat = (int64_t)ld * ld;
     if (squarings < 0) {
         double *colsum = psm;
         for (int b = blockIdx.x; b < batch; b += gridDim.x) {
             for (int c = threadIdx.x; c < ld; c += blockDim.x) colsum[c] = 0.0;
             __syncthreads();
-            if (p.kappa) {
-                const double *kap = p.kappa + (int64_t)b * p.nk;
-                for (int j = threadIdx.x; j < p.nk; j += blockDim.x) {
+            if (kappa) {
+                const double *kap = kappa + (int64_t)b * nk;
+                for (int j = threadIdx.x; j < nk; j += blockDim.x) {
                     const double v = fabs(kap[j]);
-                    atomicAdd(&colsum[p.pl[j]], v);
-                    atomicAdd(&colsum[p.pr[j]], v);
+                    atomicAdd(&colsum[pl[j]], v);
+                    atomicAdd(&colsum[pr[j]], v);
                 }
             } else {
-                const double *Ab = p.Ain + (int64_t)b * mat;
+                const double *Ab = Ain + (int64_t)b * mat;
                 for (int c = threadIdx.x; c < N; c += blockDim.x) {
                     double acc = 0.0;
                     for (int r = 0; r < N; ++r) acc += fabs(Ab[(int64_t)r * ld + c]);
@@ -474,6 +486,23 @@ __global__ void __launch_bounds__(panel::PTHREADS) expm_chain_kernel(const Chain
     } else {
         grid.sync();
     }
+    return squarings;
+}
+
+__global__ void __launch_bounds__(panel::PTHREADS) expm_chain_kernel(const ChainArgs p) {
+    extern __shared__ __align__(16) double psm[];
+    cg::grid_group grid = cg::this_grid();
+    const int N = p.N, ld = p.ld, batch = p.batch;
+    const int64_t mat = (int64_t)ld * ld, sl = mat * batch;
+    double *A2 = p.ws + 0 * sl, *A3 = p.ws + 1 * sl, *A4 = p.ws + 2 * sl, *norms = p.ws + 3 * sl;
+    double *R0 = p.ws + 7 * sl, *T0 = p.ws + 8 * sl, *T1 = p.ws + 9 * sl, *A = p.ws + (int64_t)kExpmSlots * sl;
+    const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, gthreads = (int64_t)gridDim.x * blockDim.x;
+
+    // ---- phase 0: A = 0 (packed input) and, when s is ours to choose, ||sign * input_b||_1 per matrix
+    if (p.kappa)
+        for (int64_t i = gtid; i < sl; i += gthreads) A[i] = 0.0;
+    const int squarings =
+        chain_squarings(grid, p.kappa, p.pl, p.pr, p.nk, p.Ain, N, ld, batch, p.squarings, norms, psm);
     // ---- phase 1: A = sign * input / 2^s
     const double scale = p.sign * ldexp(1.0, -squarings);
     if (p.kappa) {
@@ -567,7 +596,251 @@ int expm_chain(const ChainArgs &p, cudaStream_t stream, bool *launched) {
     return OO_OK;
 }
 
+
+// ---- adjoint of the rotation: kappa_bar from L(K, Ubar), the Frechet derivative of exp at K -----------------------
+// For U = exp(-K) and a cotangent Ubar, Kbar = -L(-K)^*(Ubar) = -L(K, Ubar) (the adjoint of L(-K, .) is L(-K^T, .) and
+// K is skew), and kappa_bar_j = Kbar[l_j,r_j] - Kbar[r_j,l_j].  L(K, E) is carried through the same scaling-and-squaring
+// chain as the rotation as a dual matrix next to every product (Al-Mohy & Higham 2009): with A = K / 2^s, E_1 = E / 2^s,
+//   E2 = E_1 A + A E_1,  E3 = E2 A + A2 E_1,  E4 = E2 A2 + A2 E2,  dB_j = c_4j+1 E_1 + c_4j+2 E2 + c_4j+3 E3,
+//   Horner: (R, L) <- (R A4 + B_j, L A4 + R E4 + dB_j),   squarings: (R, L) <- (R R, R L + L R).
+// Every dual product is two GEMMs summed into one tile.  Workspace slots (ld^2 x batch each):
+//   A A2 A3 A4 | E1 E2 E3 E4 | R0 R1 | L0 L1 | T Bt (multi-launch route only) | norms (batch doubles)
+constexpr int kVjpSlots = 14;
+
+// out = scale * X on the N x N block, 0 on the padding (the caller's padding is not read into the chain)
+__global__ void scaled_block_kernel(double *__restrict__ out, const double *__restrict__ X, double scale, int N, int ld,
+                                    int64_t total) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        const int64_t e = i % ((int64_t)ld * ld);
+        const int row = (int)(e / ld), col = (int)(e % ld);
+        out[i] = (row < N && col < N) ? scale * X[i] : 0.0;
+    }
+}
+
+// kappa_bar[b][j] = -(L_b[l_j,r_j] - L_b[r_j,l_j])
+__device__ __forceinline__ void skew_gather(const double *L, const int32_t *pl, const int32_t *pr, int nk, int ld,
+                                            int64_t i, double *kbar) {
+    const int b = (int)(i / nk), j = (int)(i - (int64_t)b * nk);
+    const double *Lb = L + (int64_t)b * ld * ld;
+    const int l = pl[j], r = pr[j];
+    kbar[i] = -(Lb[(int64_t)l * ld + r] - Lb[(int64_t)r * ld + l]);
+}
+
+__global__ void skew_gather_kernel(const double *__restrict__ L, const int32_t *__restrict__ pl,
+                                   const int32_t *__restrict__ pr, int nk, int ld, int64_t total,
+                                   double *__restrict__ kbar) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < total) skew_gather(L, pl, pr, nk, ld, i, kbar);
+}
+
+struct VjpArgs {
+    const double *kappa;          // (batch, nk)
+    const int32_t *pl, *pr;
+    int nk;
+    const double *Ubar;           // (batch, ld, ld)
+    int N, ld, batch, squarings;  // squarings < 0: chosen on the device (max over the batch), as in expm_chain_kernel
+    double *ws;                   // rotation_vjp_ws_bytes(ld, batch)
+    double *kbar;                 // (batch, nk)
+};
+
+// One cooperative launch for 8 <= ld <= 256: the phases of expm_chain_kernel with the dual products beside the
+// primal ones (2, 4, then 2 per Horner step and squaring), a grid barrier between phases, the gather at the end.
+__global__ void __launch_bounds__(panel::PTHREADS) expm_frechet_chain_kernel(const VjpArgs p) {
+    extern __shared__ __align__(16) double psm[];
+    cg::grid_group grid = cg::this_grid();
+    const int N = p.N, ld = p.ld, batch = p.batch;
+    const int64_t mat = (int64_t)ld * ld, sl = mat * batch;
+    double *A = p.ws, *A2 = p.ws + sl, *A3 = p.ws + 2 * sl, *A4 = p.ws + 3 * sl;
+    double *E1 = p.ws + 4 * sl, *E2 = p.ws + 5 * sl, *E3 = p.ws + 6 * sl, *E4 = p.ws + 7 * sl;
+    double *Rs[2] = {p.ws + 8 * sl, p.ws + 9 * sl}, *Ls[2] = {p.ws + 10 * sl, p.ws + 11 * sl};
+    double *norms = p.ws + (int64_t)kVjpSlots * sl;
+    const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, gthreads = (int64_t)gridDim.x * blockDim.x;
+
+    // ---- phase 0: A = 0, s;  phase 1: A = K / 2^s, E1 = Ubar / 2^s
+    for (int64_t i = gtid; i < sl; i += gthreads) A[i] = 0.0;
+    const int squarings =
+        chain_squarings(grid, p.kappa, p.pl, p.pr, p.nk, nullptr, N, ld, batch, p.squarings, norms, psm);
+    const double scale = ldexp(1.0, -squarings);
+    for (int64_t i = gtid; i < (int64_t)batch * p.nk; i += gthreads) {
+        const int b = (int)(i / p.nk), j = (int)(i - (int64_t)b * p.nk);
+        const double v = scale * p.kappa[i];
+        double *Ab = A + (int64_t)b * mat;
+        const int l = p.pl[j], r = p.pr[j];
+        Ab[(int64_t)l * ld + r] = v;
+        Ab[(int64_t)r * ld + l] = -v;
+    }
+    for (int64_t i = gtid; i < sl; i += gthreads) {
+        const int64_t e = i % mat;
+        const int row = (int)(e / ld), col = (int)(e % ld);
+        E1[i] = (row < N && col < N) ? scale * p.Ubar[i] : 0.0;
+    }
+    grid.sync();
+
+    double c[kTaylorDegree + 1];
+#pragma unroll
+    for (int k = 0; k <= kTaylorDegree; ++k) c[k] = inv_factorial(k);
+    const int K = ld;
+    ChainProduct q[4];
+    // A2 = A A with R = B_4 = c16 I + c17 A + c18 A2;  E2 = E1 A + A E1 with L = c17 E1 + c18 E2
+    q[0] = ChainProduct{A, A, A2, A, nullptr, nullptr, 0.0, 0.0, 0.0, 0.0, Rs[0], c[16], c[17], c[18]};
+    q[1] = ChainProduct{E1, A, E2, E1, nullptr, nullptr, 0.0, 0.0, 0.0, 0.0, Ls[0], 0.0, c[17], c[18], A, E1};
+    chain_phase(q, 2, batch, N, ld, K, psm);
+    grid.sync();
+    q[0] = ChainProduct{A2, A, A3};
+    q[1] = ChainProduct{A2, A2, A4};
+    q[2] = ChainProduct{E2, A, E3, nullptr, nullptr, nullptr, 0.0, 0.0, 0.0, 0.0, nullptr, 0.0, 0.0, 0.0, A2, E1};
+    q[3] = ChainProduct{E2, A2, E4, nullptr, nullptr, nullptr, 0.0, 0.0, 0.0, 0.0, nullptr, 0.0, 0.0, 0.0, A2, E2};
+    chain_phase(q, 4, batch, N, ld, K, psm);
+    grid.sync();
+    // Horner in A4, then the squarings; R is not formed in the last phase (only L is read)
+    const int products = 4 + squarings;
+    int cur = 0;
+    for (int i = 0; i < products; ++i) {
+        const double *Rc = Rs[cur], *Lc = Ls[cur];
+        double *Rn = Rs[cur ^ 1], *Ln = Ls[cur ^ 1];
+        if (i < 4) {
+            const int j = 3 - i;
+            q[0] = ChainProduct{Lc, A4, Ln, E1, E2, E3, 0.0, c[4 * j + 1], c[4 * j + 2], c[4 * j + 3],
+                                nullptr, 0.0, 0.0, 0.0, Rc, E4};
+            q[1] = ChainProduct{Rc, A4, Rn, A, A2, A3, c[4 * j], c[4 * j + 1], c[4 * j + 2], c[4 * j + 3]};
+        } else {
+            q[0] = ChainProduct{Rc, Lc, Ln, nullptr, nullptr, nullptr, 0.0, 0.0, 0.0, 0.0, nullptr, 0.0, 0.0, 0.0,
+                                Lc, Rc};
+            q[1] = ChainProduct{Rc, Rc, Rn};
+        }
+        chain_phase(q, i + 1 < products ? 2 : 1, batch, N, ld, K, psm);
+        grid.sync();
+        cur ^= 1;
+    }
+    // ---- kappa_bar from L(K, Ubar)
+    for (int64_t i = gtid; i < (int64_t)batch * p.nk; i += gthreads) skew_gather(Ls[cur], p.pl, p.pr, p.nk, ld, i, p.kbar);
+}
+
+int frechet_chain(const VjpArgs &p, cudaStream_t stream, bool *launched) {
+    *launched = false;
+    if (p.ld > kChainMaxN || p.ld < 8 || (p.ld & 1)) return OO_OK;
+    if (reinterpret_cast<uintptr_t>(p.ws) & 15) return OO_OK;
+    static unsigned long long configured = 0;
+    static int coop[64] = {};
+    int dev = 0;
+    OO_CUDA_CHECK(cudaGetDevice(&dev));
+    if (once_per_device(configured)) {
+        OO_CUDA_CHECK(cudaFuncSetAttribute(expm_frechet_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)panel::smem_bytes(kChainMaxN, 0, 0)));
+        int v = 0;
+        OO_CUDA_CHECK(cudaDeviceGetAttribute(&v, cudaDevAttrCooperativeLaunch, dev));
+        if (dev < 64) coop[dev] = v;
+    }
+    if (dev >= 64 || !coop[dev]) return OO_OK;
+    size_t smem = panel::smem_bytes(p.ld, 0, 0);
+    if (smem < (size_t)p.ld * sizeof(double)) smem = (size_t)p.ld * sizeof(double);
+    int per_sm = 0;
+    OO_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, expm_frechet_chain_kernel, panel::PTHREADS,
+                                                                smem));
+    if (per_sm < 1) return OO_OK;
+    const int nt = (p.ld + panel::TS - 1) / panel::TS;
+    int64_t grid = (int64_t)4 * p.batch * nt * nt;                 // the widest phase: A3, A4, E3, E4
+    if (grid > (int64_t)per_sm * sm_count()) grid = (int64_t)per_sm * sm_count();
+    void *args[] = {const_cast<VjpArgs *>(&p)};
+    OO_CUDA_CHECK(cudaLaunchCooperativeKernel((const void *)expm_frechet_chain_kernel, dim3((unsigned)grid),
+                                              dim3(panel::PTHREADS), args, smem, stream));
+    OO_LAUNCH_CHECK();
+    *launched = true;
+    return OO_OK;
+}
+
+// Multi-launch route (ld < 8, ld > 256): the same chain on dgemm_small, each dual product as T = X2 Y2 (+ dB) followed
+// by X Y + T in the beta epilogue; needs the host's squaring count.
+int frechet_multi_launch(const VjpArgs &p, cudaStream_t stream) {
+    const int N = p.N, ld = p.ld, batch = p.batch, s = p.squarings;
+    const int64_t mat = (int64_t)ld * ld, sl = mat * batch;
+    double *w = p.ws;
+    double *A = w, *A2 = w + sl, *A3 = w + 2 * sl, *A4 = w + 3 * sl;
+    double *E1 = w + 4 * sl, *E2 = w + 5 * sl, *E3 = w + 6 * sl, *E4 = w + 7 * sl;
+    double *Rs[2] = {w + 8 * sl, w + 9 * sl}, *Ls[2] = {w + 10 * sl, w + 11 * sl};
+    double *T = w + 12 * sl, *Bt = w + 13 * sl;
+    const double scale = ldexp(1.0, -s);
+    int rc;
+#define GEMM(a, b, e, d)                                                                                  \
+    if ((rc = dgemm_small(0, 0, ld, ld, ld, 1.0, (a), ld, mat, (b), ld, mat, (e) ? 1.0 : 0.0, (e), ld, mat, \
+                          0.0, (d), ld, mat, batch, stream, N)))                                        \
+    return rc
+#define LINCOMB(out, c1, X1, c2, X2, c3, X3, cI) \
+    if ((rc = lincomb((out), (c1), (X1), (c2), (X2), (c3), (X3), (cI), N, ld, batch, stream))) return rc
+    OO_CUDA_CHECK(cudaMemsetAsync(A, 0, sl * sizeof(double), stream));
+    {
+        dim3 grid((unsigned)ceil_div(p.nk, 256), (unsigned)batch);
+        skew_scatter_kernel<<<grid, 256, 0, stream>>>(p.kappa, p.pl, p.pr, p.nk, ld, scale, A);     // A = K / 2^s
+        OO_LAUNCH_CHECK();
+        int blocks = (int)ceil_div(sl, 256);
+        if (blocks > 4 * sm_count()) blocks = 4 * sm_count();
+        scaled_block_kernel<<<blocks, 256, 0, stream>>>(E1, p.Ubar, scale, N, ld, sl);                // E1 = Ubar / 2^s
+        OO_LAUNCH_CHECK();
+    }
+    double c[kTaylorDegree + 1];
+    for (int k = 0; k <= kTaylorDegree; ++k) c[k] = inv_factorial(k);
+    GEMM(A, A, nullptr, A2);
+    GEMM(A2, A, nullptr, A3);
+    GEMM(A2, A2, nullptr, A4);
+    GEMM(A, E1, nullptr, T);
+    GEMM(E1, A, T, E2);
+    GEMM(A2, E1, nullptr, T);
+    GEMM(E2, A, T, E3);
+    GEMM(A2, E2, nullptr, T);
+    GEMM(E2, A2, T, E4);
+    LINCOMB(Rs[0], c[17], A, c[18], A2, 0.0, nullptr, c[16]);
+    LINCOMB(Ls[0], c[17], E1, c[18], E2, 0.0, nullptr, 0.0);
+    const int products = 4 + s;
+    int cur = 0;
+    for (int i = 0; i < products; ++i) {
+        const bool last = i + 1 == products;
+        double *Rc = Rs[cur], *Lc = Ls[cur], *Rn = Rs[cur ^ 1], *Ln = Ls[cur ^ 1];
+        if (i < 4) {
+            const int j = 3 - i;
+            LINCOMB(Bt, c[4 * j + 1], E1, c[4 * j + 2], E2, c[4 * j + 3], E3, 0.0);
+            GEMM(Rc, E4, Bt, T);
+            GEMM(Lc, A4, T, Ln);
+            if (!last) {
+                LINCOMB(Bt, c[4 * j + 1], A, c[4 * j + 2], A2, c[4 * j + 3], A3, c[4 * j]);
+                GEMM(Rc, A4, Bt, Rn);
+            }
+        } else {
+            GEMM(Lc, Rc, nullptr, T);
+            GEMM(Rc, Lc, T, Ln);
+            if (!last) GEMM(Rc, Rc, nullptr, Rn);
+        }
+        cur ^= 1;
+    }
+#undef GEMM
+#undef LINCOMB
+    const int64_t total = (int64_t)batch * p.nk;
+    skew_gather_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(Ls[cur], p.pl, p.pr, p.nk, ld, total, p.kbar);
+    OO_LAUNCH_CHECK();
+    return OO_OK;
+}
+
 }  // namespace
+
+size_t rotation_vjp_ws_bytes(int ld, int batch) {
+    return ((size_t)kVjpSlots * batch * ld * ld + batch) * sizeof(double);
+}
+
+int kappa_rotation_vjp(const double *kappa, const int32_t *pl, const int32_t *pr, int nk, int N, int ld, int batch,
+                       int squarings, const double *Ubar, double *kbar, void *ws, size_t ws_bytes,
+                       cudaStream_t stream) {
+    OO_REQUIRE(kappa && Ubar && kbar && ws && (nk == 0 || (pl && pr)));
+    OO_REQUIRE(nk >= 0 && N > 0 && ld >= N && (ld % 2) == 0 && batch > 0 && squarings >= -1 && squarings <= 64);
+    if (ws_bytes < rotation_vjp_ws_bytes(ld, batch)) return OO_ERR_WORKSPACE;
+    if (batch > 65535) return OO_ERR_UNSUPPORTED;
+    if (nk == 0) return OO_OK;                                     // no parameters: nothing to write
+    VjpArgs p{kappa, pl, pr, nk, Ubar, N, ld, batch, squarings, reinterpret_cast<double *>(ws), kbar};
+    bool launched = false;
+    const int rc = frechet_chain(p, stream, &launched);
+    if (rc || launched) return rc;
+    if (squarings < 0) return OO_ERR_UNSUPPORTED;                  // the multi-launch route needs the host's choice
+    return frechet_multi_launch(p, stream);
+}
 
 size_t rotation_ws_bytes(int ld, int batch) {
     return (size_t)(kExpmSlots + 1) * batch * ld * ld * sizeof(double);
@@ -679,6 +952,13 @@ int oo_kappa_rotation_f64(const double *kappa, const int32_t *pair_l, const int3
                           size_t ws_bytes, void *stream) {
     return oo::kappa_rotation(kappa, pair_l, pair_r, nk, N, ld, batch, squarings, U, ws, ws_bytes,
                               (cudaStream_t)stream);
+}
+
+int oo_kappa_rotation_vjp_f64(const double *kappa, const int32_t *pair_l, const int32_t *pair_r, int nk, int N,
+                              int ld, int batch, int squarings, const double *Ubar, double *kappa_bar, void *ws,
+                              size_t ws_bytes, void *stream) {
+    return oo::kappa_rotation_vjp(kappa, pair_l, pair_r, nk, N, ld, batch, squarings, Ubar, kappa_bar, ws, ws_bytes,
+                                  (cudaStream_t)stream);
 }
 
 int oo_expm_f64(const double *A, double sign, int N, int ld, int batch, int squarings, double *U,

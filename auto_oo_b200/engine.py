@@ -401,6 +401,23 @@ class HotPathEngine:
                                                    nbytes, self.stream), "kappa_rotation")
         return U
 
+    def rotation_vjp(self, kappa, Ubar, squarings=None):
+        """kappa (B, nk), Ubar (B, ld, ld) on device -> kappa_bar (B, nk): the vector-Jacobian product of
+        :meth:`rotation` for the cotangent ``Ubar = dE/dU`` (only its N x N block is read)."""
+        kappa = self.dev(kappa).reshape(-1, self.nk)
+        B = kappa.shape[0]
+        Ubar = Ubar.reshape(B, self.ld, self.ld).contiguous()
+        if squarings is None:
+            # the single-launch adjoint (8 <= ld <= 256) chooses s on the device; the multi-launch one needs it here
+            squarings = -1 if 8 <= self.ld <= self.lib.oo_expm_device_squarings_max_n() else self.squarings_for(kappa)
+        kbar = torch.empty(B, self.nk, dtype=F64, device=self.device)
+        nbytes = self.lib.oo_workspace_bytes(_lib.OO_WS_ROTATION_VJP, self.N, self.ld, 0, B)
+        ws = self.workspace("rot_vjp", nbytes)
+        self._check(self.lib.oo_kappa_rotation_vjp_f64(_p(kappa), _p(self.pair_l), _p(self.pair_r), self.nk,
+                                                       self.N, self.ld, B, int(squarings), _p(Ubar), _p(kbar),
+                                                       _p(ws), nbytes, self.stream), "kappa_rotation_vjp")
+        return kbar
+
     def mo_coeff(self, oao_mo_coeff, U=None):
         """C' = X C_oao U  (padded, batched over U; one X per evaluation for geometry batches)."""
         Coao = oao_mo_coeff if oao_mo_coeff.dim() == 3 else oao_mo_coeff[None]
@@ -879,12 +896,13 @@ class HotPathEngine:
                     "y_matrix")
         return Y
 
-    def matmul(self, A, B):
-        """A @ B for padded (ld, ld) device matrices on the small DMMA GEMM."""
+    def matmul(self, A, B, transA=False, transB=False, alpha=1.0):
+        """alpha op(A) @ op(B) for padded (ld, ld) device matrices on the small DMMA GEMM."""
         ld = self.ld
         out = torch.empty(ld, ld, dtype=F64, device=self.device)
-        self._check(self.lib.oo_dgemm_small_f64(0, 0, ld, ld, ld, 1.0, _p(A), ld, 0, _p(B), ld, 0, 0.0, 0, ld, 0,
-                                                0.0, _p(out), ld, 0, 1, self.stream), "dgemm_small")
+        self._check(self.lib.oo_dgemm_small_f64(int(transA), int(transB), ld, ld, ld, float(alpha), _p(A), ld, 0,
+                                                _p(B), ld, 0, 0.0, 0, ld, 0, 0.0, _p(out), ld, 0, 1, self.stream),
+                    "dgemm_small")
         return out
 
     # ------------------------------------------------------------------ whole evaluations

@@ -16,9 +16,11 @@ Differences a caller can observe, all deliberate:
   of a dense ``(N,N,N,N)`` tensor; ``full_hessian_to_matrix`` accepts it (and still accepts a dense
   tensor), ``OrbitalHessian.dense()`` materialises the reference's rank-4 tensor on request;
 * differentiability: energy is differentiable (to any order) in the RDMs, the gradient once in the
-  RDMs -- what ``OO_pqc`` needs (``oo_pqc.py:86-123``).  Nothing is differentiable in ``kappa`` or
-  the MO coefficients (no driver needs it; the reference's own analytic-vs-autograd tests are
-  replayed against the CPU oracle in ``tests/``).
+  RDMs -- what ``OO_pqc`` needs (``oo_pqc.py:86-123``).  ``energy_from_kappa``, ``kappa_to_mo_coeff`` and
+  ``get_transformed_mo`` are differentiable once in ``kappa`` (and the last in ``mo_coeff``) through the
+  device adjoint of ``expm(-K)`` (``oo_kappa_rotation_vjp_f64``); a second derivative in ``kappa`` raises.
+  ``energy_from_mo_coeff`` is not differentiable in ``mo_coeff``, and the batched entry points
+  (``energies_from_kappas``, ``energy_gradient_hessian``, ``OO_energy_geometries``) detach their inputs.
 """
 from __future__ import annotations
 
@@ -174,6 +176,104 @@ class _GradientFn(torch.autograd.Function):
         eng = ctx.eng
         g1, g2 = ctx.ints.fock_gradient_vjp(ctx.FI, eng.to_padded(gbar, 2))
         return g1.to(ctx.dev1), g2.to(ctx.dev2), None, None
+
+
+_SECOND_ORDER_KAPPA = ("energy_from_kappa is differentiable once in kappa; for second derivatives in kappa use "
+                       "analytic_hessian (or OrbitalHessian.matvec)")
+
+
+def _wants_grad(*xs):
+    return torch.is_grad_enabled() and any(torch.is_tensor(x) and x.requires_grad for x in xs)
+
+
+class _KappaEnergyFn(torch.autograd.Function):
+    """``energy_from_kappa`` for a kappa that requires grad: the forward is the plain evaluation (same kernels), and
+    it keeps a hold on the transformed integrals for the backward.  dE/dgamma = c1, dE/dGamma = c2 as in
+    :class:`_EnergyFn`; dE/dkappa by :class:`_KappaBarFn`."""
+
+    @staticmethod
+    def forward(ctx, kappa, one_rdm, two_rdm, oo):
+        eng = oo.engine
+        ints = oo._mo_integrals(kappa=kappa.detach())
+        c0, c1, c2 = ints.active_hamiltonian()
+        E = eng.energy(c0, c1, c2, eng.dev(one_rdm), eng.dev(two_rdm))[0]
+        ctx.oo, ctx.ints = oo, ints
+        ctx.hold = ints.hold()                       # backward reads the integrals: keep their buffer from reuse
+        ctx.c1 = c1[0].to(one_rdm.device)
+        ctx.c2 = c2[0].to(two_rdm.device)
+        ctx.save_for_backward(kappa, one_rdm, two_rdm)
+        return E.to(one_rdm.device)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        kappa, one, two = ctx.saved_tensors
+        kbar = _KappaBarFn.apply(kappa, one, two, grad_out, ctx.oo, ctx.ints) if ctx.needs_input_grad[0] else None
+        return kbar, grad_out * ctx.c1, grad_out * ctx.c2, None
+
+
+class _KappaBarFn(torch.autograd.Function):
+    """``grad_out * dE/dkappa`` at ``C' = C expm(-K)``: with the full gradient matrix G = 2 (F - F^T) at C' (its
+    act-act block included, also when those rotations are frozen), the cotangent of U is ``-U G / 2`` and the rotation's
+    adjoint (``oo_kappa_rotation_vjp_f64``) maps it to kappa.  Its own backward raises: a second derivative in kappa
+    needs the second Frechet derivative of exp, which is not implemented."""
+
+    @staticmethod
+    def forward(ctx, kappa, one_rdm, two_rdm, grad_out, oo, ints):
+        eng = oo.engine
+        kd = eng.dev(kappa).reshape(1, -1)
+        U = eng.rotation(kd)
+        G = ints.fock_gradient(eng.dev(one_rdm), eng.dev(two_rdm), want_matrix=True, want_vector=False)[3]
+        kbar = eng.rotation_vjp(kd, eng.matmul(U[0], G[0], alpha=-0.5))[0]
+        return kbar.to(device=kappa.device, dtype=kappa.dtype).reshape(kappa.shape) * grad_out.to(kappa.device)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        raise RuntimeError(_SECOND_ORDER_KAPPA)
+
+
+class _RotationFn(torch.autograd.Function):
+    """``U = expm(-K(kappa))`` (N x N); the backward is ``oo_kappa_rotation_vjp_f64``."""
+
+    @staticmethod
+    def forward(ctx, kappa, eng):
+        ctx.eng = eng
+        ctx.save_for_backward(kappa)
+        U = eng.rotation(kappa.detach().reshape(1, -1))
+        return _like(eng.from_padded(U, 2)[0], kappa)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, Ubar):
+        kappa, = ctx.saved_tensors
+        eng = ctx.eng
+        kbar = eng.rotation_vjp(kappa.detach().reshape(1, -1), eng.to_padded(Ubar, 2)[None])[0]
+        return kbar.to(device=kappa.device, dtype=kappa.dtype).reshape(kappa.shape), None
+
+
+class _TransformedMOFn(torch.autograd.Function):
+    """``M expm(-K(kappa))``; backward: ``Mbar = Outbar U^T``, ``Ubar = M^T Outbar`` -> ``oo_kappa_rotation_vjp_f64``."""
+
+    @staticmethod
+    def forward(ctx, mo_coeff, kappa, eng):
+        U = eng.rotation(kappa.detach().reshape(1, -1))[0]
+        M = eng.to_padded(mo_coeff, 2)
+        ctx.eng, ctx.U, ctx.M = eng, U, M
+        ctx.save_for_backward(mo_coeff, kappa)
+        return _like(eng.from_padded(eng.matmul(M, U)[None], 2)[0], mo_coeff)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, out_bar):
+        mo_coeff, kappa = ctx.saved_tensors
+        eng = ctx.eng
+        ob = eng.to_padded(out_bar, 2)
+        mbar = kbar = None
+        if ctx.needs_input_grad[0]:
+            mbar = _like(eng.from_padded(eng.matmul(ob, ctx.U, transB=True)[None], 2)[0], mo_coeff)
+        if ctx.needs_input_grad[1]:
+            kbar = eng.rotation_vjp(kappa.detach().reshape(1, -1), eng.matmul(ctx.M, ob, transA=True)[None])[0]
+            kbar = kbar.to(device=kappa.device, dtype=kappa.dtype).reshape(kappa.shape)
+        return mbar, kbar, None
 
 
 class PendingEvaluation:
@@ -400,14 +500,20 @@ class OO_energy:
         return skew_symmetric_to_vector(kappa_matrix)[self.params_idx]
 
     def kappa_to_mo_coeff(self, kappa):
-        """``expm(-K(kappa))`` (reference ``oo_energy.py:226-230``) by ``oo_kappa_rotation_f64``."""
+        """``expm(-K(kappa))`` (reference ``oo_energy.py:226-230``) by ``oo_kappa_rotation_f64``; differentiable in a
+        ``kappa`` tensor (backward: ``oo_kappa_rotation_vjp_f64``)."""
         eng = self.engine
+        if _wants_grad(kappa):
+            return _RotationFn.apply(kappa, eng)
         U = eng.rotation(_as_tensor(kappa).detach().reshape(1, -1))
         return _like(eng.from_padded(U, 2)[0], kappa)
 
     def get_transformed_mo(self, mo_coeff, kappa):
-        """``mo_coeff @ expm(-K)`` (reference ``oo_energy.py:232-236``)."""
+        """``mo_coeff @ expm(-K)`` (reference ``oo_energy.py:232-236``); differentiable in a ``kappa`` tensor and in
+        a ``mo_coeff`` tensor (a numpy ``mo_coeff`` gives a numpy result, without a gradient)."""
         eng = self.engine
+        if torch.is_tensor(mo_coeff) and torch.is_tensor(kappa) and _wants_grad(mo_coeff, kappa):
+            return _TransformedMOFn.apply(mo_coeff, kappa, eng)
         U = eng.rotation(_as_tensor(kappa).detach().reshape(1, -1))
         out = eng.matmul(eng.to_padded(_as_tensor(mo_coeff), 2), U[0])
         return _like(eng.from_padded(out[None], 2)[0], mo_coeff)
@@ -441,13 +547,18 @@ class OO_energy:
         return _EnergyFn.apply(one, two, self.engine, c0, c1, c2)
 
     def energy_from_kappa(self, kappa, one_rdm, two_rdm):
-        """Energy at ``C' = C expm(-K(kappa))`` (reference ``oo_energy.py:199-202``)."""
+        """Energy at ``C' = C expm(-K(kappa))`` (reference ``oo_energy.py:199-202``).  Differentiable in the RDMs
+        (to any order) and, for a ``kappa`` tensor that requires grad, once in ``kappa``: the gradient comes back on
+        ``kappa``'s device and dtype; a second derivative in ``kappa`` raises ``RuntimeError``."""
+        if _wants_grad(kappa):
+            return _KappaEnergyFn.apply(kappa, _as_tensor(one_rdm), _as_tensor(two_rdm), self)
         c0, c1, c2 = self._mo_integrals(kappa=_as_tensor(kappa).detach()).active_hamiltonian()
         return _EnergyFn.apply(_as_tensor(one_rdm), _as_tensor(two_rdm), self.engine, c0, c1, c2)
 
     def energies_from_kappas(self, kappas, one_rdm, two_rdm):
         """``energy_from_kappa`` for a batch ``kappas (B, n_kappa)`` in one pass (batched launches);
-        returns ``(B,)`` on the device of ``kappas``.  Used by the speculative line search."""
+        returns ``(B,)`` on the device of ``kappas``.  Used by the speculative line search.  Not differentiable:
+        ``kappas`` and the RDMs are detached."""
         eng = self.engine
         kappas = _as_tensor(kappas).detach().reshape(-1, self.n_kappa)
         run = eng.evaluate_graphed if self.cuda_graphs else eng.evaluate
@@ -739,7 +850,8 @@ class OO_energy_geometries:
 
     ``mols``: sequence of duck-typed ``Moldata_pyscf`` objects; ``oao_mo_coeff``: ``(G, N, N)`` (or
     one ``(N, N)`` matrix used for all).  ``energy_gradient_hessian(kappa, one_rdm, two_rdm)`` takes
-    ``kappa (G, n_kappa)`` and RDMs shared ``(na,na)/(na^4)`` or per geometry ``(G, ...)``."""
+    ``kappa (G, n_kappa)`` and RDMs shared ``(na,na)/(na^4)`` or per geometry ``(G, ...)``.  Its results are not
+    differentiable: ``kappa`` and the RDMs are detached."""
 
     def __init__(self, mols, ncas, nelecas, oao_mo_coeff, freeze_active=False, device=None,
                  eri_symmetry="auto", cuda_graphs="auto"):

@@ -59,8 +59,9 @@ enum {
     OO_WS_HESSIAN_VECTOR  = 11, /* oo_hessian_vector_f64: pass N = na (!), nI = no+na, batch = nv   */
     OO_WS_HESSIAN_DIAGONAL = 12, /* oo_hessian_diagonal_f64 (nI = no+na); oo_class_hessian_diagonal_f64
                                    needs no workspace                                              */
-    OO_WS_KRYLOV = 13          /* oo_davidson_expand_f64 / oo_pcg_step_f64: pass N = n (vector length), nI = k
+    OO_WS_KRYLOV = 13,         /* oo_davidson_expand_f64 / oo_pcg_step_f64: pass N = n (vector length), nI = k
                                   (largest basis, <= 64), ld = batch = 1                                        */
+    OO_WS_ROTATION_VJP = 14    /* oo_kappa_rotation_vjp_f64                                                      */
 };
 
 int         oo_abi_version(void);
@@ -154,6 +155,17 @@ int oo_kappa_rotation_f64(const double *kappa, const int32_t *pair_l, const int3
 /* largest N for which `squarings` = -1 is accepted: 256 (64 with the environment variable
  * OO_OPT_EXPM_MULTI_LAUNCH, 0 with OO_OPT_EXPM_UNFUSED; both kept for A/B tests)       */
 int oo_expm_device_squarings_max_n(void);
+
+/* kappa_bar[b][j] = Kbar[l_j,r_j] - Kbar[r_j,l_j],  Kbar = -L(K(kappa_b), Ubar_b):  the VJP of
+ * oo_kappa_rotation_f64 (same kappa / pair / squarings conventions), i.e. what autograd of the reference's
+ * kappa -> expm(-K) (oo_energy.py:213-236) returns for the cotangent Ubar = dE/dU.  L(K, E) is the Frechet derivative
+ * of exp at K, carried as a dual matrix through the rotation's Taylor / squaring chain.  8 <= ld <= 256: one
+ * cooperative launch, `squarings` = -1 lets it choose s on the device (max over the batch); other ld: a multi-launch
+ * chain that needs squarings >= 0.  Only the N x N block of Ubar[b] (ld x ld) is read.  Repeats are bit-identical.
+ * ws: oo_workspace_bytes(OO_WS_ROTATION_VJP, N, ld, 0, batch).                                                  */
+int oo_kappa_rotation_vjp_f64(const double *kappa, const int32_t *pair_l, const int32_t *pair_r,
+                              int nk, int N, int ld, int batch, int squarings,
+                              const double *Ubar, double *kappa_bar, void *ws, size_t ws_bytes, void *stream);
 
 /* expm(sign * A) of arbitrary (not nec. skew) ld x ld matrices with ||A||_1 <= 0.95 * 2^squarings */
 int oo_expm_f64(const double *A, double sign, int N, int ld, int batch, int squarings,
